@@ -29,6 +29,14 @@ exchange is one all-gather of the 96 B commitments per layer).
 iteration runs one operation of each kind of each layer AT FULL SIZE and the step is those times multiplied by the op
 counts (`extrapolated_by_op_counts`); nothing is rescaled from smaller sizes, warm-up iterations never feed the value.
 The default arm never touches oracle/ outside its `cpu_baseline` leg.
+
+--dump-outputs DIR writes what the last timed step computed, for comparing two builds output for output (the inputs are seeded, so
+they are the same on every run with the same arguments): `<layer>_commitments.npy`, every job's commitment of every layer as affine
+(x, y) (identity = (0, 0)), and `<last layer>_coefficients.npy`, the coefficient vectors of the last layer's transform chains, which
+stay in device memory after the step, at the rows of `<last layer>_coefficient_rows.npy` (a fixed, seeded sample).  Field elements
+are canonical integers as eight little-endian 32-bit limbs in float64, which is exact.  Earlier layers' coefficient vectors are
+overwritten by the later layers of the same step, and the extended (coset) evaluations go to a ring of buffers that the jobs reuse,
+so neither is dumped.
 """
 from __future__ import annotations
 
@@ -48,6 +56,9 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 MAC32_PER_MADD = 1280  # 10 modmul x 128 MAC32 (SURVEY.md §8(d))
+Q_MOD = 0x30644E72E131A029B85045B68181585D97816A916871CA8D3C208C16D87CFD47  # BN254 base field
+R_MOD = 0x30644E72E131A029B85045B68181585D2833E84879B9709143E1F593F0000001  # BN254 scalar field
+DUMP_COEFF_BYTES = 32 << 20  # cap on the sampled coefficient rows of --dump-outputs (8 float64 limbs = 64 B per element)
 
 # name, k, witness-like Lagrange columns, uniform Lagrange columns, coefficient-form commits, extra coset NTTs
 Layer = namedtuple("Layer", "name k wit uni coeff extra")
@@ -289,6 +300,36 @@ def run_reference(args):
 # ====================================================================================================
 # product arm
 # ====================================================================================================
+def _limbs32(values) -> np.ndarray:
+    """integers below 2^256 as rows of eight little-endian 32-bit limbs in float64 (exact)"""
+    return np.array([[(v >> (32 * i)) & 0xFFFFFFFF for i in range(8)] for v in values], dtype=np.float64).reshape(-1, 8)
+
+
+def dump_outputs(out_dir, plans, pool_coeff, suffix=""):
+    """--dump-outputs: the commitments of every layer and a seeded sample of the last layer's coefficient vectors (see the module
+    docstring); called right after the timed steps, while the buffers still hold the last step's results."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    mont = lambda limbs, mod: int.from_bytes(limbs.tobytes(), "little") * pow(1 << 256, -1, mod) % mod
+    for pl in plans:
+        xy = []
+        for c in pl.get("commits", np.zeros((0, 12), np.uint64)):  # Jacobian (X, Y, Z), Montgomery form
+            x, y, z = (mont(c[4 * i:4 * i + 4], Q_MOD) for i in range(3))
+            zi = pow(z, -1, Q_MOD) if z else 0
+            xy += [x * zi * zi % Q_MOD, y * zi * zi * zi % Q_MOD]
+        np.save(os.path.join(out_dir, f"{pl['layer'].name}_commitments{suffix}.npy"), _limbs32(xy).reshape(-1, 2, 8))
+    last = plans[-1]
+    n, chains = last["n"], len(last["nt"])
+    if chains:
+        rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, 1 << 16, DUMP_COEFF_BYTES // (64 * chains)), replace=False))
+        coeff = pool_coeff[:chains * n * 4].view(chains, n, 4)[:, torch.from_numpy(rows).to(pool_coeff.device)]
+        coeff = coeff.cpu().numpy().view(np.uint64).reshape(-1, 4)
+        name = last["layer"].name
+        np.save(os.path.join(out_dir, f"{name}_coefficients{suffix}.npy"), _limbs32(mont(e, R_MOD) for e in coeff).reshape(chains, -1, 8))
+        np.save(os.path.join(out_dir, f"{name}_coefficient_rows{suffix}.npy"), rows.astype(np.float64))
+
+
 def run_b200(args):
     import torch
 
@@ -444,9 +485,10 @@ def run_b200(args):
     def run_layer(pl, key):
         jl = pl[key]
         if jl:
-            commits[: len(jl)] = zk.run_column_jobs(ctx, jl, pl["layer"].k, omega_inv=pl["dom"].omega_inv,
-                                                    extended_omega=pl["dom"].extended_omega,
-                                                    extended_omega_inv=pl["dom"].extended_omega_inv, extended_k=pl["ek"])
+            pl["commits"] = zk.run_column_jobs(ctx, jl, pl["layer"].k, omega_inv=pl["dom"].omega_inv,
+                                               extended_omega=pl["dom"].extended_omega,
+                                               extended_omega_inv=pl["dom"].extended_omega_inv, extended_k=pl["ek"])
+            commits[: len(jl)] = pl["commits"]
         torch.cuda.current_stream().synchronize()
         if dist:  # the next proof hashes this proof's commitments: one tiny all-gather per layer, the only exchange
             t = torch.zeros((world, gather_cap, 12), dtype=torch.int64, device=dev)
@@ -507,6 +549,8 @@ def run_b200(args):
         sampler.start()
     sec, wall, _, launches = timed("resident", args.steps, args.warmup, profile=False)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, plans, pool_coeff, f"_rank{rank}" if world > 1 else "")
     per_layer_value = [sum(v) / len(v) / 1e3 for v in layer_ms["resident"]]
     # per-kernel durations (roofline, kernel_ms_per_step) come from a separate profiled pass of the SAME step with the
     # two-stream overlap switched off: while kernels of two streams share the SMs their individual durations say nothing
@@ -630,6 +674,7 @@ def main():
     ap.add_argument("--only", default="", help="profiling: restrict the chunk step to these layers, e.g. inner or layer1,layer2")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only (ncu): device-resident arm only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -105,3 +108,27 @@ def test_reference_arm_of_the_chunk_step_is_built_from_full_size_samples_only():
         total += det[n]["layer_s"]
     assert abs(total - d["sample_values_s"][-1]) < 1e-9
     assert "configs[2]" in d["config"]["workload"] and "shrunk" in d["metric"]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_whatever_the_step_count(tmp_path):
+    """--dump-outputs writes float arrays (64 MB at most) of the last timed step; the inputs are seeded, so 1 and 3 timed steps
+    dump the same values, and --steps sets the number of timed steps (3 steps launch 3 times the kernels of 1)."""
+    dumps, launches = [], []
+    for steps in (1, 3):
+        d = tmp_path / f"steps{steps}"
+        r = run("--shrink", "8", "--steps", str(steps), "--warmup", "1", "--no-cpu-baseline", "--skip-e2e", "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+        assert line["steps"] == steps
+        launches.append(line["gpu_launches"])
+        dumps.append({f.name: np.load(f) for f in sorted(d.iterdir())})
+    a, b = dumps
+    assert set(a) == {"inner_commitments.npy", "layer1_commitments.npy", "layer2_commitments.npy", "layer2_coefficients.npy",
+                      "layer2_coefficient_rows.npy"}
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for name, v in a.items():
+        assert v.dtype in (np.float32, np.float64) and np.array_equal(v, b[name]), name
+    assert a["inner_commitments.npy"].shape == (416 + 96 + 6 + 1, 2, 8) and a["layer2_commitments.npy"].any()
+    assert a["layer2_coefficients.npy"].shape[0] == 5 and a["layer2_coefficients.npy"].any()
+    assert launches[1] == 3 * launches[0] > 0

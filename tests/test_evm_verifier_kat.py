@@ -1,26 +1,23 @@
 """The reference's EVM verifier PROGRAM run on the reference's shipped proof (SURVEY.md §8(c) fixture 3, §8(f).4; the `verifier
-bytecode check` of BASELINE configs[4]): release-v0.13.1/evm_verifier.yul (the Yul source of evm_verifier.bin) is interpreted
-statement by statement (tests/yul_verifier.py) on calldata = proof.data with pi.data spliced in after the 12 accumulator limbs (the layer-6 EVM proof).  It must accept,
-and must reject when a byte of the proof or of the public input is flipped.  The deployed artefact itself, evm_verifier.bin, is
-run too: a small stack machine (tests/evm_bytecode.py) executes its constructor, takes the 13 987-byte runtime it returns and
-calls it with the same calldata -- same verdicts, same precompile and Keccak call counts as the Yul source.
+bytecode check` of BASELINE configs[4]): the deployed artefact release-v0.13.1/evm_verifier.bin is run by a small stack machine
+(tests/evm_bytecode.py), which executes its constructor, takes the 13 987-byte runtime it returns and calls it with calldata =
+proof.data with pi.data spliced in after the 12 accumulator limbs (the layer-6 EVM proof).  It must accept, with the precompile
+and Keccak call counts the program's Yul source (evm_verifier.yul) has on the same calldata, and must reject when a byte of the
+proof or of the public input is flipped.  The artefacts and the Yul run's counts are stored under tests/golden.
 
 The elliptic-curve precompiles (ecAdd 0x06, ecMul 0x07, ecPairing 0x08) are served twice: by the independent big-integer model
 and by the PRODUCT's host-side code (csrc/ec.cuh group law + pairing_bn254.hpp, through tests/host_emul/libpairing_host.so) --
 so the product's verifier-side arithmetic is held to a complete real proof of the reference, not only to its accumulator.
-CPU only; reads the reference tree, so it is skipped where /root/reference does not exist."""
+CPU only."""
 import ctypes as C
 import os
 import subprocess
 
-import pytest
-
 from pairing_model import Q, g1_add, g1_mul, pairing_check
-from yul_verifier import keccak256, verify
+from reference_data import GOLD, REL
+from yul_verifier import keccak256
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REL = "/root/reference/release-v0.13.1"
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REL, "evm_verifier.yul")), reason="reference tree not present")
 
 
 def be(v):
@@ -93,11 +90,10 @@ def h_add_mul(lib):
 
 
 def load():
-    yul = open(os.path.join(REL, "evm_verifier.yul")).read()
     pi, proof = open(os.path.join(REL, "pi.data"), "rb").read(), open(os.path.join(REL, "proof.data"), "rb").read()
-    # the reference's own test assembles the calldata like this (/root/reference/integration/tests/unit_tests.rs:30-32,
+    # the reference's own test assembles the calldata like this (integration/tests/unit_tests.rs:30-32,
     # `proof.splice(384..384, pi)`): the 12 accumulator limbs, the 13 public-input words, then the proof proper
-    return yul, proof[:384] + pi + proof[384:]
+    return proof[:384] + pi + proof[384:]
 
 
 def test_keccak256_known_answers():
@@ -106,28 +102,7 @@ def test_keccak256_known_answers():
     assert keccak256(bytes(200)).hex() != keccak256(bytes(201)).hex()  # multi-block inputs absorb every block
 
 
-def test_reference_verifier_program_accepts_the_shipped_proof_on_the_bigint_model():
-    yul, calldata = load()
-    assert len(calldata) == 416 + 1632
-    ok, m = verify(yul, calldata, m_add, m_mul, m_pairing)
-    assert ok
-    assert m.precompile_calls[8] == 1 and m.precompile_calls[6] > 10 and m.precompile_calls[7] > 10 and m.keccak_calls >= 9
-
-
-def test_reference_verifier_program_on_the_products_host_curve_and_pairing_code():
-    yul, calldata = load()
-    add, mul, pairing = h_add_mul(host_lib())
-    ok, m = verify(yul, calldata, add, mul, pairing)
-    assert ok and m.precompile_calls[8] == 1
-    # a flipped byte anywhere -- a public input, a commitment, an evaluation, the last opening point -- is rejected
-    for pos in (40, 384 + 5, 800 + 5, 800 + 700, len(calldata) - 3):
-        bad = bytearray(calldata)
-        bad[pos] ^= 1
-        ok2, _ = verify(yul, bytes(bad), add, mul, pairing)
-        assert not ok2, pos
-
-
-# ---- the deployed bytecode itself (evm_verifier.bin), not only its Yul source
+# ---- the deployed bytecode (evm_verifier.bin)
 def load_bin():
     return open(os.path.join(REL, "evm_verifier.bin"), "rb").read()
 
@@ -135,24 +110,27 @@ def load_bin():
 def test_reference_verifier_bytecode_deploys_and_accepts_the_shipped_proof():
     from evm_bytecode import call, deploy
 
-    _, calldata = load()
+    calldata = load()
+    assert len(calldata) == 416 + 1632
     runtime = deploy(load_bin())
     assert len(runtime) == 0x36A3  # the size the constructor pushes before CODECOPY
     ok, m = call(runtime, calldata, m_add, m_mul, m_pairing)
     assert ok
     # same work as the Yul source does: one pairing, the same EC and hash call counts
-    _, y = verify(load()[0], calldata, m_add, m_mul, m_pairing)
-    assert m.precompile_calls == y.precompile_calls and m.keccak_calls == y.keccak_calls
+    y = GOLD["evm_verifier_yul_run"]
+    assert y["accepted"] and m.precompile_calls[8] == 1
+    assert m.precompile_calls == {int(a): n for a, n in y["precompile_calls"].items()} and m.keccak_calls == y["keccak_calls"]
 
 
 def test_reference_verifier_bytecode_on_the_products_host_curve_and_pairing_code():
     from evm_bytecode import call, deploy
 
-    _, calldata = load()
+    calldata = load()
     runtime = deploy(load_bin())
     add, mul, pairing = h_add_mul(host_lib())
     ok, m = call(runtime, calldata, add, mul, pairing)
     assert ok and m.precompile_calls[8] == 1
+    # a flipped byte anywhere -- a public input, a commitment, an evaluation, the last opening point -- is rejected
     for pos in (40, 384 + 5, 800 + 5, 800 + 700, len(calldata) - 3):
         bad = bytearray(calldata)
         bad[pos] ^= 1
@@ -164,7 +142,7 @@ def test_reference_verifier_bytecode_on_the_products_host_curve_and_pairing_code
 
 
 # ---- the PRODUCT's EVMVerifier (scroll-prover_b200/evm_verifier_b200.hpp): the same bytecode on a C++ stack machine whose
-# precompiles are the product's host curve / pairing code -- /root/reference/integration/src/verifier.rs without an EVM
+# precompiles are the product's host curve / pairing code -- the reference's integration/src/verifier.rs without an EVM
 EVM_SRC = os.path.join(ROOT, "tests", "cpp", "test_evm_verifier.cpp")
 EVM_BIN = os.path.join(ROOT, "tests", "cpp", "test_evm_verifier")
 
@@ -186,7 +164,7 @@ def test_the_products_evm_verifier_accepts_the_shipped_proof_like_the_python_mac
     from evm_bytecode import call, deploy
 
     verdict, info = product_evm()
-    _, calldata = load()
+    calldata = load()
     ok, m = call(deploy(load_bin()), calldata, m_add, m_mul, m_pairing)
     assert verdict == "ACCEPT" and ok
     assert int(info["runtime_bytes"]) == 0x36A3 and int(info["steps"]) == m.steps  # instruction for instruction

@@ -1,6 +1,6 @@
 """The product-side reader of snark-verifier `*.protocol` files (scroll-prover_b200/protocol_json.hpp, SURVEY.md §8(f).3) against
-Python's own reading of the same JSON: on a small synthetic protocol (always) and on the reference's shipped
-release-v0.13.1/chunk.protocol (where the reference tree exists): the domain equals the C++ mirror's EvaluationDomain::new_(5, 25),
+Python's own reading of the same JSON: on a small synthetic protocol and on the reference's shipped
+release-v0.13.1/chunk.protocol (stored under tests/golden): the domain equals the C++ mirror's EvaluationDomain::new_(5, 25),
 the 7 preprocessed commitments equal the points of vk_chunk.vkey as serde_bn254.hpp decodes them, and the proof size implied by
 the protocol (5 witness commitments + 4 quotient chunks + 17 evaluations + 2 SHPLONK points) is the 896 bytes of the reference's
 chunk proofs (integration/tests/test_data/full_proof_1.json)."""
@@ -8,12 +8,11 @@ import json
 import os
 import subprocess
 
-import pytest
+from reference_data import REL
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.path.join(ROOT, "tests", "cpp", "test_protocol_json.cpp")
 BIN = os.path.join(ROOT, "tests", "cpp", "test_protocol_json")
-REL = "/root/reference/release-v0.13.1"
 
 
 def binary():
@@ -74,7 +73,6 @@ def test_synthetic_protocol(tmp_path):
     assert rc == 1 and "unknown polynomial" in out["error"]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REL, "chunk.protocol")), reason="reference tree not present")
 def test_reference_chunk_protocol_matches_the_mirror_and_the_shipped_vk():
     rc, out = run(os.path.join(REL, "chunk.protocol"), os.path.join(REL, "vk_chunk.vkey"))
     assert rc == 0

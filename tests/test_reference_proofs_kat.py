@@ -1,5 +1,5 @@
 """The reference's OWN proofs verified offline (SURVEY.md §8(c) fixture 4): the chunk proofs (layer 2, k = 25, 896 bytes) and the
-batch proofs (layer 4, k = 26) shipped under /root/reference/integration/tests/test_data are read with the protocol JSON they carry,
+batch proofs (layer 4, k = 26) shipped in the reference's integration/tests/test_data are read with the protocol JSON they carry,
 their Poseidon transcript is replayed, the quotient identity is evaluated from the protocol's expression tree, the SHPLONK (Bdfg21)
 opening is folded into a KZG accumulator and the accumulator is decided against the trusted setup's G2 constants
 (release-v0.13.1/evm_verifier.yul:1230-1239) -- tests/snark_verifier_model.py, a big-integer model of snark-verifier's native
@@ -8,20 +8,18 @@ accumulator each proof carries in its instances must be valid as well, and a fli
 
 What this pins: the proof format the hot path's outputs end up in -- compressed commitments, evaluation order, rotation sets, the
 powers of mu / gamma (= the `y` / `v` of halo2's ProverSHPLONK, ascending, which scroll-prover_b200/plonk_b200.hpp follows) --
-against real proofs of the reference, not against our own reading of it.  CPU only; skipped where the reference tree is absent."""
+against real proofs of the reference, not against our own reading of it.  CPU only; the proofs are the sample stored in
+tests/golden/reference_proofs.json (tests/reference_data.py)."""
 import base64
 import ctypes as C
-import glob
 import json
 import os
 
-import pytest
-
 from pairing_model import G2_GEN, pairing_check
+from reference_data import GOLD, REL, proof_files_dir
 from snark_verifier_model import PoseidonSpec, verify_plonk
 
-DATA = "/root/reference/integration/tests/test_data"
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(DATA, "full_proof_1.json")), reason="reference tree not present")
+DATA = proof_files_dir()
 
 # -[s]G2 of the degree-26 SRS as the EVM verifier holds it (evm_verifier.yul:1236-1239; EIP-197 word order x_c1, x_c0, y_c1, y_c0)
 NEG_S_G2 = ((0x17944351223333f260ddc3b4af45191b856689eda9eab5cbcddbbe570ce860d2, 0x186282957db913abd99f91db59fe69922e95040603ef44c0bd7aa3adeef8f5ac),
@@ -48,13 +46,8 @@ def decide(lhs, rhs):
 
 
 def chunk_entries():
-    out = []
-    for name, take in (("full_proof_1.json", 1), ("batch-task-no-encode.json", 1), ("batch-task-with-blob-raw.json", 4),
-                       ("batch-task-with-blob.json", 2), ("full_proof_batch_prove_1.json", 1)):
-        out += [(name, i, e) for i, e in enumerate(json.load(open(os.path.join(DATA, name)))["chunk_proofs"][:take])]
-    first = sorted(glob.glob(os.path.join(DATA, "batch_tasks", "*.json")))[0]
-    out += [(os.path.basename(first), i, e) for i, e in enumerate(json.load(open(first))["chunk_proofs"][:2])]
-    return out
+    """(file, index, proof object) of every stored chunk proof"""
+    return [(name, i, e) for name in GOLD["files"] for i, e in enumerate(json.load(open(os.path.join(DATA, name))).get("chunk_proofs", []))]
 
 
 def test_poseidon_constants_reproduce_the_published_t3_parameters():
@@ -67,8 +60,8 @@ def test_poseidon_constants_reproduce_the_published_t3_parameters():
 
 def test_reference_chunk_proofs_verify():
     entries = chunk_entries()
-    assert len(entries) == 11
-    release = json.load(open("/root/reference/release-v0.13.1/chunk.protocol"))
+    assert len(entries) == 8
+    release = json.load(open(os.path.join(REL, "chunk.protocol")))
     for name, i, e in entries:
         proto, proof, instances = decode(e)
         assert len(proof) == 896 and proto["domain"]["k"] == 25 and proto["quotient"]["num_chunk"] == 4 and len(instances[0]) == 44, (name, i)
@@ -126,7 +119,7 @@ def test_oracle_multiexp_redoes_the_msms_of_real_proofs_and_the_reference_srs_ac
         return O.fq_to_int(a[:4]), O.fq_to_int(a[4:])
 
     picks = [decode(json.load(open(os.path.join(DATA, "full_proof_1.json")))["chunk_proofs"][0]),
-             decode(chunk_entries()[5][2]),
+             decode(json.load(open(os.path.join(DATA, "batch-task-with-blob-raw.json")))["chunk_proofs"][3]),
              decode(json.load(open(os.path.join(DATA, "full_proof_batch_agg_1.json"))))]
     for proto, proof, instances in picks:
         lhs, rhs, info = verify_plonk(proto, instances, proof, SPEC)

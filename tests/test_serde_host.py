@@ -105,21 +105,20 @@ def test_random_points_round_trip_and_agree_with_the_oracle(lib):
     assert parities == {0, 1}
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/release-v0.13.1/evm_verifier.yul"), reason="reference tree not present")
 def test_vk_bundle_points_are_the_constants_the_evm_verifier_hard_codes(lib):
     """Two artefacts of the reference tied together by OUR codec: the seven compressed commitments of release-v0.13.1/vk_bundle.vkey,
     decompressed (square root + sign bit) by the product's serde_bn254.hpp and by the oracle, are exactly the uncompressed (x, y)
-    words the generated EVM verifier stores for its fixed / permutation commitments (evm_verifier.yul)."""
-    import re
-
+    words the generated EVM verifier pushes (PUSH32) for its fixed / permutation commitments (evm_verifier.bin)."""
     from oracle import oracle as O
+    from reference_data import REL
 
-    raw = open("/root/reference/release-v0.13.1/vk_bundle.vkey", "rb").read()
-    consts = {int(m, 16) for m in re.findall(r"0x[0-9a-f]{64}", open("/root/reference/release-v0.13.1/evm_verifier.yul").read())}
+    raw = bytes.fromhex(GOLD["files"]["vk_bundle.vkey"]["hex"])
+    code = open(os.path.join(REL, "evm_verifier.bin"), "rb").read()
+    pushed = lambda v: b"\x7f" + v.to_bytes(32, "big") in code
     ok, _, _, _, pts, _ = read_vk(lib, raw)
     assert ok == 1 and len(pts) == 7
     for i, p in enumerate(pts):
         x, y = O.fq_to_int(p[:4]), O.fq_to_int(p[4:])
-        assert x in consts and y in consts, i
+        assert pushed(x) and pushed(y), i
         assert np.array_equal(O.g1_decompress(raw[8 + 32 * i:40 + 32 * i]), p)
-        assert (0x30644E72E131A029B85045B68181585D97816A916871CA8D3C208C16D87CFD47 - y) not in consts  # the other square root is not in the program: the sign bit matters
+        assert not pushed(0x30644E72E131A029B85045B68181585D97816A916871CA8D3C208C16D87CFD47 - y)  # the other square root is not in the program: the sign bit matters

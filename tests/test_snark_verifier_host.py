@@ -1,13 +1,13 @@
 """The product's host-side verifier for the reference's proof format (scroll-prover_b200/snark_verifier_b200.hpp: PlonkVerifier +
 PoseidonTranscript + Bdfg21 + KZG decider, C++ mirror of snark-verifier @ 948671c as scroll-prover's ChunkVerifier / BatchVerifier use
-it, /root/reference/integration/src/prove.rs:50-53,78-80):
+it, integration/src/prove.rs:50-53,78-80 of the reference):
 
   * it ACCEPTS the reference's shipped chunk proofs (k = 25) and batch proofs (k = 26) from the protocol JSON, instances and proof
     bytes alone -- the same decisions as the independent big-integer model (tests/snark_verifier_model.py);
   * it rejects tampered proofs, wrong public inputs, a corrupted carried accumulator and another trusted setup;
   * it ACCEPTS the proofs our own create_proof makes with the Poseidon transcript (plonk_b200.hpp) under the exported protocol --
     i.e. prover and verifier of the product meet in the reference's format.
-CPU only.  The reference-proof cases are skipped where the reference tree is absent."""
+CPU only.  The reference's proofs are the sample stored in tests/golden/reference_proofs.json (tests/reference_data.py)."""
 import base64
 import json
 import os
@@ -16,12 +16,12 @@ import subprocess
 import pytest
 
 from pairing_model import Q
+from reference_data import GOLD, REL, proof_files_dir
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.path.join(ROOT, "tests", "cpp", "test_snark_verifier.cpp")
 BIN = os.path.join(ROOT, "tests", "cpp", "test_snark_verifier")
-DATA = "/root/reference/integration/tests/test_data"
-have_ref = pytest.mark.skipif(not os.path.exists(os.path.join(DATA, "full_proof_1.json")), reason="reference tree not present")
+DATA = proof_files_dir()
 NEG_S_G2 = ((0x17944351223333f260ddc3b4af45191b856689eda9eab5cbcddbbe570ce860d2, 0x186282957db913abd99f91db59fe69922e95040603ef44c0bd7aa3adeef8f5ac),
             (0x06ecdb9f9567f59ed2eee36e1e1d58797fd13cc97fafc2910f5e8a12f202fa9a, 0x06d971ff4a7467c3ec596ed6efc674572e32fd6f52b721f97e35b0b3d3546753))
 S_G2 = (NEG_S_G2[0], ((-NEG_S_G2[1][0]) % Q, (-NEG_S_G2[1][1]) % Q))
@@ -51,7 +51,6 @@ def decode(entry):
     return json.loads(base64.b64decode(entry["protocol"])), base64.b64decode(entry["proof"]), [[int.from_bytes(raw[i:i + 32], "big") for i in range(0, len(raw), 32)]]
 
 
-@have_ref
 def test_reference_chunk_and_batch_proofs_are_accepted(tmp_path):
     from test_reference_proofs_kat import chunk_entries
 
@@ -62,10 +61,9 @@ def test_reference_chunk_and_batch_proofs_are_accepted(tmp_path):
     for name in ("full_proof_batch_agg_1.json", "full_proof_batch_agg_2.json"):
         assert verdict(tmp_path, *decode(json.load(open(os.path.join(DATA, name))))) == "ACCEPT", name
         n += 1
-    assert n == 13
+    assert n == 10
 
 
-@have_ref
 def test_tampering_is_rejected(tmp_path):
     proto, proof, instances = decode(json.load(open(os.path.join(DATA, "full_proof_1.json")))["chunk_proofs"][0])
     for pos in (3, 200, 300, 500, 850, 895):
@@ -104,26 +102,23 @@ def verify_file(path, s_g2=S_G2, tamper=False):
     return accepted, total, lines[:-1]
 
 
-@have_ref
 def test_every_proof_file_the_reference_ships_is_read_and_accepted():
     """scroll-prover_b200/proof_files.hpp reads the reference's proof files AS WRITTEN (serde_json objects with base64 fields, the
-    chunk_proofs containers of batch tasks) and runs verify_chunk_proof / verify_batch_proof on every proof object in them: all 319
-    distinct chunk proofs of the batch tasks and both batch proofs are accepted -- the protocol they carry, the proof, the carried
+    chunk_proofs containers of batch tasks) and runs verify_chunk_proof / verify_batch_proof on every proof object in them: the 8
+    stored chunk proofs (of the reference's 319) and both batch proofs are accepted -- the protocol they carry, the proof, the carried
     accumulator, and the vk bytes beside them matching the protocol's preprocessed commitments."""
-    import glob
-
-    files = sorted(glob.glob(os.path.join(DATA, "*.json"))) + sorted(glob.glob(os.path.join(DATA, "batch_tasks", "*.json")))
+    files = [os.path.join(DATA, name) for name in GOLD["files"]]
     chunk = batch = 0
     for f in files:
         accepted, total, lines = verify_file(f)
         assert accepted == total and total >= 1, (f, [l for l in lines if not l.startswith("ACCEPT")][:3])
         chunk += sum(1 for l in lines if l.startswith("ACCEPT chunk k=25 proof_bytes=896"))
         batch += sum(1 for l in lines if l.startswith("ACCEPT batch k=26"))
-    assert (chunk, batch) == (319, 2)
+    assert (chunk, batch) == (8, 2)
     # and every one of those chunk proofs was made for the RELEASED circuit: the vk and the protocol it carries are byte-for-byte
     # release-v0.13.1/vk_chunk.vkey and chunk.protocol (four different git versions of the prover among them)
-    rel_vk = open("/root/reference/release-v0.13.1/vk_chunk.vkey", "rb").read()
-    rel_proto = json.load(open("/root/reference/release-v0.13.1/chunk.protocol"))
+    rel_vk = open(os.path.join(REL, "vk_chunk.vkey"), "rb").read()
+    rel_proto = json.load(open(os.path.join(REL, "chunk.protocol")))
     versions = set()
     for f in files:
         for cp in json.load(open(f)).get("chunk_proofs", []):
@@ -132,7 +127,6 @@ def test_every_proof_file_the_reference_ships_is_read_and_accepted():
     assert len(versions) == 4
 
 
-@have_ref
 def test_proof_files_with_a_flipped_proof_byte_or_another_setup_are_rejected(tmp_path):
     f = os.path.join(DATA, "batch-task-with-blob-raw.json")
     assert verify_file(f)[:2] == (4, 4)
@@ -161,7 +155,6 @@ def test_keccak256_of_the_proof_file_reader_known_answers():
     assert subprocess.run([binary(), "--keccak", ""], capture_output=True, text=True).stdout.strip() == "c5d2460186f7233c927e7db2dcc703c0e500b653ca82273b7bfad8045d85a470"
 
 
-@have_ref
 def test_a_chunk_proof_is_bound_to_the_chunk_info_beside_it(tmp_path):
     """instances[12..44] = keccak256(chain_id || prev_state_root || post_state_root || withdraw_root || data_hash || keccak256(tx_bytes)):
     true for every shipped chunk proof (test_every_proof_file_... goes through the same check); any changed field is refused"""
@@ -178,7 +171,6 @@ def test_a_chunk_proof_is_bound_to_the_chunk_info_beside_it(tmp_path):
     assert verify_file(p)[:2] == (1, 1)
 
 
-@have_ref
 def test_a_batch_proof_carries_its_batch_hash_and_the_second_continues_the_first(tmp_path):
     b1, b2 = (json.load(open(os.path.join(DATA, f"full_proof_batch_agg_{i}.json"))) for i in (1, 2))
     w1, w2 = decode(b1)[2][0], decode(b2)[2][0]
@@ -197,31 +189,28 @@ def batch_task(path):
     return out.split()[0], fields, out
 
 
-@have_ref
 def test_batch_tasks_are_consistent_and_their_header_hashes_chain(tmp_path):
     """proof_files.hpp reads the reference's batch proving tasks (chunk_infos + chunk_proofs + batch_header): every chunk info is the
     one its proof carries, state roots chain, header.data_hash = keccak(chunk data hashes); BatchHeader::batch_hash (keccak of the
-    193-byte encoding) is pinned by the reference's data twice: the ten consecutive tasks 293205..293214 chain through
-    parent_batch_hash, and the header of full_proof_batch_prove_1.json hashes to the batch_hash of the batch proof made from it."""
-    import glob
-
-    tasks = sorted(glob.glob(os.path.join(DATA, "batch_tasks", "*.json")))
-    assert len(tasks) == 10
-    prev, total = None, 0
-    for f in tasks:
-        verdict, info, out = batch_task(f)
-        assert verdict == "CONSISTENT", out
+    193-byte encoding) is pinned by the reference's data twice: the headers of the ten consecutive tasks 293205..293214 chain through
+    parent_batch_hash, and the header of full_proof_batch_prove_1.json hashes to the batch_hash of the batch proof made from it.
+    Of those ten tasks only the headers are stored: a header without chunks is still hashed, and the task is refused."""
+    p = tmp_path / "task.json"
+    prev = None
+    for index, header in sorted(GOLD["batch_headers"].items()):
+        p.write_text(json.dumps({"chunk_infos": [], "chunk_proofs": [], "batch_header": header}))
+        verdict, info, out = batch_task(p)
+        assert verdict == "INCONSISTENT" and "one chunk info per chunk proof" in out and info["chunks"] == "0", out
         if prev is not None:
-            assert info["parent"] == prev, f
+            assert info["parent"] == prev, index
         prev = info["batch_hash"]
-        total += int(info["chunks"])
-    assert total == 289
-    for name in ("batch-task-no-encode.json", "batch-task-with-blob-raw.json", "batch-task-with-blob.json"):
-        assert batch_task(os.path.join(DATA, name))[0] == "CONSISTENT", name
+    assert len(GOLD["batch_headers"]) == 10
+    raw = os.path.join(DATA, "batch-task-with-blob-raw.json")
+    verdict, info, out = batch_task(raw)
+    assert verdict == "CONSISTENT" and info["chunks"] == "4", out
     # the batch proof full_proof_batch_agg_1.json was made from the task full_proof_batch_prove_1.json: same batch hash
     j = json.load(open(os.path.join(DATA, "full_proof_batch_prove_1.json")))
     j["chunk_infos"] = [cp["chunk_info"] for cp in j["chunk_proofs"]]
-    p = tmp_path / "task.json"
     p.write_text(json.dumps(j))
     verdict, info, out = batch_task(p)
     assert verdict == "CONSISTENT"
@@ -229,15 +218,15 @@ def test_batch_tasks_are_consistent_and_their_header_hashes_chain(tmp_path):
     agg = os.path.join(DATA, "full_proof_batch_agg_1.json")
     out = subprocess.run([binary(), "--batch-task", str(p), agg], capture_output=True, text=True, timeout=120).stdout
     assert "proof_matches_task=1" in out
-    out = subprocess.run([binary(), "--batch-task", tasks[0], agg], capture_output=True, text=True, timeout=120).stdout
+    out = subprocess.run([binary(), "--batch-task", raw, agg], capture_output=True, text=True, timeout=120).stdout
     assert "proof_matches_task=0" in out
     assert "0x" + info["batch_hash"] == json.load(open(os.path.join(DATA, "full_proof_batch_agg_1.json")))["batch_hash"], out
     # inconsistencies are named
-    t = json.load(open(tasks[0]))
+    t = json.load(open(raw))
     t["chunk_infos"][3]["post_state_root"] = t["chunk_infos"][3]["post_state_root"][:-1] + ("0" if t["chunk_infos"][3]["post_state_root"][-1] != "0" else "1")
     p.write_text(json.dumps(t))
     assert batch_task(p)[0] == "INCONSISTENT"
-    t = json.load(open(tasks[0]))
+    t = json.load(open(raw))
     t["chunk_infos"], t["chunk_proofs"] = t["chunk_infos"][:-1], t["chunk_proofs"][:-1]
     p.write_text(json.dumps(t))
     verdict, _, out = batch_task(p)
