@@ -310,6 +310,29 @@ B200ZK_API int32_t b200zk_graph_evaluate_rows(b200zk_ctx* ctx, const b200zk_grap
  * 32-byte elements over NVLink, on the context stream).  world must divide 2^log_size (a power of two); world == 1 is a no-op. */
 B200ZK_API int32_t b200zk_allgather_rows(b200zk_ctx* ctx, void* values_dev, uint32_t log_size);
 
+/* ---- the extended coset by parts ------------------------------------------------------------------
+ * With n = 2^k, J = 2^(extended_k - k) (1 <= k, k <= extended_k <= 28, J <= 16), the extended coset point of row t = r + J*i is
+ * zeta * w_ext^t = g_r * w^i, g_r = zeta * w_ext^r (w_ext^J = w).  So the extended domain is J disjoint parts of n points:
+ * rotations stay inside a part, X^n - 1 is the constant g_r^n - 1 on part r, and a quotient can be built part by part with
+ * n-element columns only.  Same bytes as the full-coset entries. */
+/* out_dev[j][i] = p_j(g_part * w^i), i < 2^k: element part + J*i of coeff_to_extended(p_j).  coeffs[j]: 2^k coefficients,
+ * host or device; out_dev[j]: device. */
+B200ZK_API int32_t b200zk_coeff_to_extended_parts(b200zk_ctx* ctx, const void* const* coeffs, uint32_t count, uint32_t k,
+                                                  uint32_t extended_k, uint32_t part, void* const* out_dev);
+/* b200zk_graph_evaluate on the 2^k rows of one part: columns hold that part's values, a rotation reads row (i + rot) mod 2^k,
+ * B200ZK_SRC_EXTENDED_X is g_part * w^i, PreviousValue is the old values[i].  values_dev: 2^k elements (device). */
+B200ZK_API int32_t b200zk_graph_evaluate_part(b200zk_ctx* ctx, const b200zk_graph* graph, const void* const* fixed_dev,
+                                              uint32_t n_fixed, const void* const* advice_dev, uint32_t n_advice,
+                                              const void* const* instance_dev, uint32_t n_instance, const void* challenges32,
+                                              uint32_t n_challenges, const void* beta32, const void* gamma32, const void* theta32,
+                                              const void* y32, uint32_t k, uint32_t extended_k, uint32_t part, void* values_dev);
+/* parts_dev: 2^extended_k elements, part-major (part r at r * 2^k); consumed (used as scratch).  out_dev receives n_pieces * 2^k
+ * coefficients (1 <= n_pieces <= J): extended_to_coeff of the interleaved vector (first passed through divide_by_vanishing_poly
+ * when divide_by_vanishing != 0), truncated.  out_dev may equal parts_dev.  With world | J, a rank's
+ * b200zk_shard_range(2^extended_k) slice is whole parts, so b200zk_allgather_rows(ctx, parts_dev, extended_k) completes it. */
+B200ZK_API int32_t b200zk_extended_parts_to_coeff(b200zk_ctx* ctx, void* parts_dev, uint32_t k, uint32_t extended_k,
+                                                  uint32_t n_pieces, int divide_by_vanishing, void* out_dev);
+
 /* ---- diagnostics ----------------------------------------------------------------------------- */
 /* element-wise Fr/Fq Montgomery product of two arrays on the device (field-layer parity tests) */
 B200ZK_API int32_t b200zk_debug_field_op(b200zk_ctx* ctx, int field /*0 Fr,1 Fq*/, int op /*0 mul,1 add,2 sub,3 inv*/,

@@ -84,6 +84,23 @@ pub(crate) fn extended_to_coeff(values: &mut [Fr], extended_k: u32, extended_ome
     check(unsafe { sys::b200zk_ntt_fr(ctx(), values.as_mut_ptr() as _, extended_k, p(&extended_omega_inv), 1, sys::COSET_POST) });
 }
 
+/// The extended coset by parts (part r = the n points zeta * w_ext^r * w^i): p(zeta * w_ext^part * w^i) for every column, into
+/// device buffers of n elements each (the caller keeps them resident, e.g. from b200zk_buf_alloc).
+pub(crate) fn coeff_to_extended_parts(columns: &[&[Fr]], k: u32, extended_k: u32, part: u32, out_dev: &[*mut c_void]) {
+    assert!(columns.iter().all(|c| c.len() == 1 << k));
+    assert_eq!(columns.len(), out_dev.len());
+    let ptrs: Vec<*const c_void> = columns.iter().map(|c| c.as_ptr() as *const c_void).collect();
+    check(unsafe {
+        sys::b200zk_coeff_to_extended_parts(ctx(), ptrs.as_ptr(), ptrs.len() as u32, k, extended_k, part, out_dev.as_ptr())
+    });
+}
+/// divide_by_vanishing_poly (optional) + extended_to_coeff + truncate to n_pieces * n, from the J parts laid out part-major in
+/// one device buffer of 2^extended_k elements (consumed); the pieces land in `out_dev` (may be `parts_dev`).
+pub(crate) fn extended_parts_to_coeff(parts_dev: *mut c_void, k: u32, extended_k: u32, n_pieces: u32, divide_by_vanishing: bool,
+                                      out_dev: *mut c_void) {
+    check(unsafe { sys::b200zk_extended_parts_to_coeff(ctx(), parts_dev, k, extended_k, n_pieces, divide_by_vanishing as c_int, out_dev) });
+}
+
 pub(crate) fn eval_polynomial(poly: &[Fr], point: Fr) -> Fr {
     let mut out = Fr::zero();
     check(unsafe { sys::b200zk_eval_poly(ctx(), poly.as_ptr() as _, poly.len() as u64, p(&point), &mut out as *mut Fr as _) });

@@ -111,6 +111,10 @@ def _load():
         "b200zk_graph_evaluate_rows": [vp, vp, C.POINTER(vp), u32, C.POINTER(vp), u32, C.POINTER(vp), u32, vp, u32, vp, vp, vp, vp, vp,
                                        vp, u32, i32, u64, u64],
         "b200zk_allgather_rows": [vp, vp, u32],
+        "b200zk_coeff_to_extended_parts": [vp, C.POINTER(vp), u32, u32, u32, u32, C.POINTER(vp)],
+        "b200zk_graph_evaluate_part": [vp, vp, C.POINTER(vp), u32, C.POINTER(vp), u32, C.POINTER(vp), u32, vp, u32, vp, vp, vp, vp, u32,
+                                       u32, u32, vp],
+        "b200zk_extended_parts_to_coeff": [vp, vp, u32, u32, u32, C.c_int, vp],
         "b200zk_debug_field_op": [vp, C.c_int, C.c_int, vp, vp, vp, u64],
         "b200zk_profile_enable": [vp, C.c_int],
         "b200zk_profile_reset": [vp],
@@ -136,7 +140,7 @@ ABI_SYMBOLS = [
     "b200zk_g1_generator_mul_batch", "b200zk_fft_g1", "b200zk_g_to_lagrange", "b200zk_ntt_fr", "b200zk_ntt_fr_ext", "b200zk_ctx_set_overlap", "b200zk_run_column_jobs", "b200zk_commit_columns", "b200zk_poly_add", "b200zk_poly_sub",
     "b200zk_poly_mul", "b200zk_poly_scale", "b200zk_poly_axpy", "b200zk_eval_poly", "b200zk_inner_product", "b200zk_batch_invert",
     "b200zk_kate_division", "b200zk_prefix_scan", "b200zk_poly_lincomb", "b200zk_permutation_product", "b200zk_logup_running_sum", "b200zk_graph_create", "b200zk_graph_check",
-    "b200zk_graph_destroy", "b200zk_graph_info", "b200zk_graph_evaluate", "b200zk_graph_evaluate_rows", "b200zk_allgather_rows", "b200zk_debug_field_op", "b200zk_profile_enable", "b200zk_profile_reset", "b200zk_profile_read", "b200zk_msm_set_window", "b200zk_msm_last_stats", "b200zk_msm_total_adds",
+    "b200zk_graph_destroy", "b200zk_graph_info", "b200zk_graph_evaluate", "b200zk_graph_evaluate_rows", "b200zk_allgather_rows", "b200zk_coeff_to_extended_parts", "b200zk_graph_evaluate_part", "b200zk_extended_parts_to_coeff", "b200zk_debug_field_op", "b200zk_profile_enable", "b200zk_profile_reset", "b200zk_profile_read", "b200zk_msm_set_window", "b200zk_msm_last_stats", "b200zk_msm_total_adds",
 ]
 
 _lib = None
@@ -664,6 +668,23 @@ class Graph:
                                                  log_size, rot_scale))
         return values
 
+    def evaluate_part(self, values, k: int, extended_k: int, part: int, fixed=(), advice=(), instance=(), challenges=None, beta=None,
+                      gamma=None, theta=None, y=None):
+        """The same on the 2^k rows of part `part` of the extended coset (b200zk_graph_evaluate_part): columns hold that part's
+        values (EvaluationDomain.coeff_to_extended_parts), rotations wrap within the part."""
+        assert _count(values, 32) == 1 << k
+        zero = np.zeros(4, np.uint64)
+        tf, kf = Context._dev_table(fixed)
+        ta, ka = Context._dev_table(advice)
+        ti, ki = Context._dev_table(instance)
+        ch = np.ascontiguousarray(np.asarray(challenges if challenges is not None else [], dtype=np.uint64).reshape(-1, 4))
+        sc = [_ptr(zero if v is None else v) for v in (beta, gamma, theta, y)]
+        pv, kv = _ptr(values)
+        self.ctx._ck(lib().b200zk_graph_evaluate_part(self.ctx._h, self._h, tf, len(fixed), ta, len(advice), ti, len(instance),
+                                                      C.c_void_p(ch.ctypes.data) if len(ch) else None, len(ch), *[p for p, _ in sc], k,
+                                                      extended_k, part, pv))
+        return values
+
     def release(self):
         if self._h:
             lib().b200zk_graph_destroy(self.ctx._h, self._h)
@@ -791,3 +812,28 @@ class EvaluationDomain:
         """ifft(extended_omega_inv) + distribute_powers_zeta(out of coset); returns the first n*(j-1) coefficients."""
         self.ctx.best_fft(a, self.extended_omega_inv, self.extended_k, inverse_scale=True, coset_mode=COSET_POST)
         return a[: self.n * self.quotient_poly_degree]
+
+    @property
+    def n_parts(self) -> int:
+        """J = 2^(extended_k - k): the extended coset is J parts of n points, part r = zeta * extended_omega^r * <omega>."""
+        return 1 << (self.extended_k - self.k)
+
+    def coeff_to_extended_parts(self, coeffs, part: int, outs):
+        """outs[j][i] = coeffs[j](zeta * extended_omega^part * omega^i): coeff_to_extended(coeffs[j])[part::J] (outs: CUDA tensors)."""
+        assert len(coeffs) == len(outs)
+        assert all(_count(c, 32) == self.n for c in coeffs) and all(_count(o, 32) == self.n for o in outs)
+        ti, ki = Context._dev_table(coeffs)
+        to, ko = Context._dev_table(outs)
+        self.ctx._ck(lib().b200zk_coeff_to_extended_parts(self.ctx._h, ti, len(coeffs), self.k, self.extended_k, part, to))
+        return outs
+
+    def extended_parts_to_coeff(self, parts, divide_by_vanishing: bool = False, n_pieces: int | None = None, out=None):
+        """parts: CUDA tensor of 2^extended_k elements, part-major (consumed).  Returns n_pieces * n coefficients (default
+        n_pieces = quotient_poly_degree): extended_to_coeff of the interleaved vector, after divide_by_vanishing_poly if asked."""
+        assert _count(parts, 32) == 1 << self.extended_k
+        n_pieces = self.quotient_poly_degree if n_pieces is None else n_pieces
+        out = parts if out is None else out
+        pp, kp = _ptr(parts)
+        po, ko = _ptr(out)
+        self.ctx._ck(lib().b200zk_extended_parts_to_coeff(self.ctx._h, pp, self.k, self.extended_k, n_pieces, int(divide_by_vanishing), po))
+        return out[: n_pieces * self.n]

@@ -416,6 +416,54 @@ int32_t b200zk_ntt_fr(b200zk_ctx* ctx, void* data, uint32_t log_n, const void* o
     return b200zk_ntt_fr_ext(ctx, data, log_n, data, log_n, omega32, inverse_scale, coset_mode);
 }
 
+// ---- the extended coset by parts (DESIGN.md "Quotient construction") ----------------------------
+int32_t b200zk_coeff_to_extended_parts(b200zk_ctx* ctx, const void* const* coeffs, uint32_t count, uint32_t k, uint32_t extended_k,
+                                       uint32_t part, void* const* out_dev) {
+    CHECK_CTX(ctx);
+    B2_TRY(check_part_args(ctx, "coeff_to_extended_parts", k, extended_k, part));
+    if (count && (!coeffs || !out_dev)) return fail(ctx, B200ZK_E_INVALID, "coeff_to_extended_parts: null pointer table");
+    Guard g(ctx);
+    for (uint32_t j = 0; j < count; ++j) {
+        if (!coeffs[j]) return fail(ctx, B200ZK_E_INVALID, "coeff_to_extended_parts: coeffs[%u] is null", j);
+        if (!out_dev[j] || !is_device_ptr(out_dev[j]))
+            return fail(ctx, B200ZK_E_INVALID, "coeff_to_extended_parts: out[%u] must be a device pointer", j);
+    }
+    const size_t bytes = sizeof(Fr) << k;
+    for (uint32_t j = 0; j < count; ++j) {
+        const void* in_dev = nullptr;
+        B2_TRY(stage_in(ctx, ctx->stage_in, coeffs[j], bytes, &in_dev));  // stream order keeps the staging buffer's reuse safe
+        B2_TRY(ntt_part_run(ctx, (const Fr*)in_dev, (Fr*)out_dev[j], k, extended_k, part, false, Fr::one()));
+    }
+    return B200ZK_OK;
+}
+
+int32_t b200zk_extended_parts_to_coeff(b200zk_ctx* ctx, void* parts_dev, uint32_t k, uint32_t extended_k, uint32_t n_pieces,
+                                       int divide_by_vanishing, void* out_dev) {
+    CHECK_CTX(ctx);
+    B2_TRY(check_part_args(ctx, "extended_parts_to_coeff", k, extended_k, 0));
+    const uint32_t log_j = extended_k - k, J = 1u << log_j;
+    if (n_pieces < 1 || n_pieces > J)
+        return fail(ctx, B200ZK_E_INVALID, "extended_parts_to_coeff: n_pieces = %u must lie in [1, J = %u]", n_pieces, J);
+    Guard g(ctx);
+    if (!parts_dev || !is_device_ptr(parts_dev)) return fail(ctx, B200ZK_E_INVALID, "extended_parts_to_coeff: parts must be a device pointer");
+    if (!out_dev || !is_device_ptr(out_dev)) return fail(ctx, B200ZK_E_INVALID, "extended_parts_to_coeff: out must be a device pointer");
+    const uint64_t n = 1ull << k;
+    // part r: g_r^n = zeta^n w_J^r, w_J = w_ext^n the primitive J-th root; divide_by_vanishing_poly is 1 / (g_r^n - 1) on the part
+    Fr zeta_n = Fr::one(), zeta = host_zeta();
+    for (uint64_t i = 0; i < n % 3; ++i) zeta_n = zeta_n * zeta;  // zeta^3 = 1
+    const Fr w_j = host_root_of_unity(log_j);
+    Fr g_n = zeta_n;
+    for (uint32_t r = 0; r < J; ++r, g_n = g_n * w_j) {
+        Fr scale = divide_by_vanishing ? (g_n - Fr::one()).inv() : Fr::one();
+        Fr* p = (Fr*)parts_dev + (uint64_t)r * n;
+        B2_TRY(ntt_part_run(ctx, p, p, k, extended_k, r, true, scale));
+    }
+    Fr jf = Fr::zero();
+    jf.l.v[0] = J;
+    const Fr j_inv = jf.to_mont().inv();
+    return parts_recombine_run(ctx, (const Fr*)parts_dev, k, log_j, n_pieces, zeta_n.inv(), w_j.inv(), j_inv, (Fr*)out_dev);
+}
+
 // ---- device-resident column pipeline (SURVEY.md §8(f).1) -------------------------------------------
 static int32_t pipeline_init(b200zk_ctx* ctx) {
     if (ctx->copy_stream) return B200ZK_OK;

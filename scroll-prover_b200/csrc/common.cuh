@@ -267,5 +267,24 @@ Fr host_zeta();
 int32_t comm_destroy(b200zk_ctx* ctx);  // comm.cu
 int32_t ntt_run(b200zk_ctx* ctx, const Fr* in, uint32_t log_in, Fr* out, uint32_t log_n, const Fr& omega,
                 int inverse_scale, int coset_mode);
+Fr host_root_of_unity(uint32_t log_n);  // EvaluationDomain's primitive 2^log_n-th root
+int32_t ntt_part_run(b200zk_ctx* ctx, const Fr* in, Fr* out, uint32_t k, uint32_t ext_k, uint32_t part, bool inverse,
+                     const Fr& scale);
+int32_t parts_recombine_run(b200zk_ctx* ctx, const Fr* parts, uint32_t k, uint32_t log_j, uint32_t n_pieces, const Fr& zeta_n_inv,
+                            const Fr& w_j_inv, const Fr& j_inv, Fr* out);  // quotient.cu
+
+// the extended domain of 2^extended_k points split into J = 2^(extended_k - k) parts of 2^k points (the coset-part entries)
+constexpr uint32_t MAX_PART_LOG = 4;  // J <= 16
+inline int32_t check_part_args(b200zk_ctx* ctx, const char* what, uint32_t k, uint32_t extended_k, uint32_t part) {
+    if (k < 1) return fail(ctx, B200ZK_E_INVALID, "%s: k = %u, must be at least 1", what, k);
+    if (extended_k < k || extended_k > 28)
+        return fail(ctx, B200ZK_E_INVALID, "%s: extended_k = %u must lie in [k, 28] (k = %u)", what, extended_k, k);
+    if (extended_k - k > MAX_PART_LOG)
+        return fail(ctx, B200ZK_E_INVALID, "%s: J = 2^%u parts exceeds the supported maximum of %u", what, extended_k - k,
+                    1u << MAX_PART_LOG);
+    if (part >= (1u << (extended_k - k)))
+        return fail(ctx, B200ZK_E_INVALID, "%s: part %u >= J = %u", what, part, 1u << (extended_k - k));
+    return B200ZK_OK;
+}
 
 }  // namespace b200zk

@@ -18,6 +18,10 @@
 // shared by every domain size under the same root (w_{2^u} = ROOT_OF_UNITY^(2^(28-u)) for all k).
 // Fused: zero padding + zeta^i coset pre-scaling on load (coeff_to_extended), n^-1 and zeta^-i
 // post-scaling on the final store (ifft / extended_to_coeff).
+// Part transforms (ntt_part_run, DESIGN.md "Quotient construction") are separate instantiations (Tw = PartTwist) that
+// also scale by w_ext^(part*i) on load or by its inverse on store; the plain instantiations (Tw = NoTwist) are unchanged.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace b200zk {
@@ -46,6 +50,18 @@ __device__ __forceinline__ Fr sel3(const Fr3& t, uint32_t r) {  // no dynamic in
     return o;
 }
 
+// The twist of part r of the extended coset: element i is scaled by u^(r*i mod 2^ext_k), u = w_ext on a forward transform's
+// load and u = w_ext^-1 on an inverse transform's store.  u^e comes from the level-ext_k run of the universal twiddle table
+// of u's family (u^j for j < 2^(ext_k-1); the upper half by u^(j + 2^(ext_k-1)) = -u^j), the table that coeff_to_extended /
+// extended_to_coeff keep anyway and whose level-k run is also the n-point transform's: no per-part table is built.
+struct NoTwist {};
+struct PartTwist {
+    const Fr* wtab;   // u^j, j < 2^(ext_k - 1)
+    uint64_t mask;    // 2^ext_k - 1
+    uint64_t part;
+    int pre, post;
+};
+
 struct LevelRoots {
     Fr w[29];  // w[u] = primitive 2^u-th root
 };
@@ -65,6 +81,12 @@ __device__ __forceinline__ Fr ldg_fr(const Fr* p) {
     r.l.v[0] = a.x; r.l.v[1] = a.y; r.l.v[2] = a.z; r.l.v[3] = a.w;
     r.l.v[4] = b.x; r.l.v[5] = b.y; r.l.v[6] = b.z; r.l.v[7] = b.w;
     return r;
+}
+__device__ __forceinline__ Fr part_root(const PartTwist& tw, uint64_t e) {  // u^e, e <= mask
+    const uint64_t half = (tw.mask + 1) >> 1;
+    Fr w = ldg_fr(tw.wtab + (e & (half - 1)));
+    if (e >= half) w = Fr::zero() - w;
+    return w;
 }
 __device__ __forceinline__ void st_fr(Fr* p, const Fr& r) {
     uint4* q = reinterpret_cast<uint4*>(p);
@@ -104,10 +126,11 @@ __global__ void ntt_build_table(Fr* tab, LevelRoots roots, uint32_t log_n) {
 }
 
 // One pass over one tile.  C = lanes per tile (8, or 1 for the single-pass small transform).
-template <int C, bool LAST>
+template <int C, bool LAST, class Tw = NoTwist>
 __global__ void __launch_bounds__(NTT_THREADS, 3)
 ntt_pass_kernel(const Fr* __restrict__ in, Fr* __restrict__ out, const Fr* __restrict__ tab, NttPass ps, Fr3 pre_c,
-                Fr3 post_c) {
+                Fr3 post_c, Tw tw) {
+    constexpr bool TWIST = !std::is_same<Tw, NoTwist>::value;
     extern __shared__ uint4 smem[];
     const uint32_t m = ps.m, L = 1u << m, E = L * C;
     uint4* lo = smem;
@@ -180,6 +203,12 @@ ntt_pass_kernel(const Fr* __restrict__ in, Fr* __restrict__ out, const Fr* __res
             if (ps.p == 0 && ps.pre) {
                 uint32_t r3 = (uint32_t)(gi % 3);
                 if (r3) v = v * sel3(pre_c, r3);
+            }
+            if constexpr (TWIST) {
+                if (ps.p == 0 && tw.pre) {
+                    const uint64_t e = (tw.part * gi) & tw.mask;
+                    if (e) v = v * part_root(tw, e);
+                }
             }
         }
         uint32_t pos = __brev(d) >> (32 - m);
@@ -268,6 +297,12 @@ ntt_pass_kernel(const Fr* __restrict__ in, Fr* __restrict__ out, const Fr* __res
         } else {
             go = ((uint64_t)K << t) + c + lane;
             if (ps.post) v = v * sel3(post_c, (uint32_t)(go % 3));
+            if constexpr (TWIST) {
+                if (tw.post) {
+                    const uint64_t e = (tw.part * go) & tw.mask;
+                    if (e) v = v * part_root(tw, e);
+                }
+            }
         }
         st_fr(out + go, v);
     }
@@ -363,14 +398,15 @@ static void plan_digits(uint32_t log_n, uint32_t* P, uint32_t dig[4]) {
     for (uint32_t i = 0; i < 4; ++i) dig[i] = (i < p) ? basebits + (i < extra ? 1 : 0) : 0;
 }
 
-template <int C, bool LAST>
+template <int C, bool LAST, class Tw>
 static int32_t launch_pass(b200zk_ctx* ctx, const Fr* in, Fr* out, const Fr* tab, const NttPass& ps, const Fr3& pre_c,
-                           const Fr3& post_c) {
+                           const Fr3& post_c, const Tw& tw) {
     uint32_t L = 1u << ps.m, E = L * C;
     size_t smem = (size_t)(2 * E + (LAST ? 0 : 2 * L)) * sizeof(uint4);
-    const uint32_t optin_bit = 1u << ((C == 8 ? 0 : 2) + (LAST ? 1 : 0));
+    // bits 0-3: plain instantiations, bits 9-12: part-twist instantiations (bit 8 is the graph kernel's)
+    const uint32_t optin_bit = 1u << ((C == 8 ? 0 : 2) + (LAST ? 1 : 0) + (std::is_same<Tw, NoTwist>::value ? 0 : 9));
     if (!(ctx->smem_optin & optin_bit)) {
-        B2_CUDA(ctx, cudaFuncSetAttribute(ntt_pass_kernel<C, LAST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        B2_CUDA(ctx, cudaFuncSetAttribute(ntt_pass_kernel<C, LAST, Tw>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           (int)((2 * (1u << NTT_MAX_DIGIT) * C + 2 * (1u << NTT_MAX_DIGIT)) * sizeof(uint4))));
         ctx->smem_optin |= optin_bit;
     }
@@ -379,9 +415,48 @@ static int32_t launch_pass(b200zk_ctx* ctx, const Fr* in, Fr* out, const Fr* tab
     uint32_t threads = nb >= NTT_THREADS ? NTT_THREADS : (nb < 32 ? 32 : nb);
     {
         ProfScope psc(ctx, PROF_NTT_PASS);
-        ntt_pass_kernel<C, LAST><<<(uint32_t)tiles, threads, smem, ctx->stream>>>(in, out, tab, ps, pre_c, post_c);
+        ntt_pass_kernel<C, LAST, Tw><<<(uint32_t)tiles, threads, smem, ctx->stream>>>(in, out, tab, ps, pre_c, post_c, tw);
     }
     B2_LAUNCH_CHECK(ctx);
+    return B200ZK_OK;
+}
+
+// the pass sequence of one transform: a single pass up to 2^8 elements, else P passes through ctx->ntt_work
+template <class Tw>
+static int32_t ntt_passes(b200zk_ctx* ctx, const Fr* in, uint32_t log_in, Fr* out, uint32_t log_n, const Fr* tab, int pre, int post,
+                          const Fr3& pre_c, const Fr3& post_c, const Tw& tw) {
+    NttPass ps;
+    memset(&ps, 0, sizeof ps);
+    ps.log_n = log_n;
+    plan_digits(log_n, &ps.P, ps.dig);
+    if (ps.P == 1) {
+        ps.p = 0;
+        ps.t = 0;
+        ps.m = log_n;
+        ps.rest = 0;
+        ps.log_in = log_in;
+        ps.pre = pre;
+        ps.post = post;
+        return launch_pass<1, true>(ctx, in, out, tab, ps, pre_c, post_c, tw);
+    }
+    size_t bytes = sizeof(Fr) << log_n;
+    B2_TRY(scratch_reserve(ctx, ctx->ntt_work, bytes));
+    Fr* W = (Fr*)ctx->ntt_work.p;
+    uint32_t t = 0;
+    for (uint32_t p = 0; p < ps.P; ++p) {
+        ps.p = p;
+        ps.t = t;
+        ps.m = ps.dig[p];
+        ps.rest = log_n - t - ps.m;
+        ps.log_in = (p == 0) ? log_in : log_n;
+        ps.pre = (p == 0) ? pre : 0;
+        ps.post = (p + 1 == ps.P) ? post : 0;
+        if (p + 1 < ps.P)
+            B2_TRY((launch_pass<8, false>(ctx, p == 0 ? in : W, W, tab, ps, pre_c, post_c, tw)));
+        else
+            B2_TRY((launch_pass<8, true>(ctx, W, out, tab, ps, pre_c, post_c, tw)));
+        t += ps.m;
+    }
     return B200ZK_OK;
 }
 
@@ -408,42 +483,46 @@ int32_t ntt_run(b200zk_ctx* ctx, const Fr* in, uint32_t log_in, Fr* out, uint32_
     post_c.c[0] = scale;
     post_c.c[1] = (coset_mode == B200ZK_COSET_POST) ? scale * zeta2 : scale;
     post_c.c[2] = (coset_mode == B200ZK_COSET_POST) ? scale * zeta : scale;
-
-    NttPass ps;
-    memset(&ps, 0, sizeof ps);
-    ps.log_n = log_n;
-    plan_digits(log_n, &ps.P, ps.dig);
     const int pre = (coset_mode == B200ZK_COSET_PRE), post = (inverse_scale || coset_mode == B200ZK_COSET_POST);
+    return ntt_passes(ctx, in, log_in, out, log_n, tab, pre, post, pre_c, post_c, NoTwist{});
+}
 
-    if (ps.P == 1) {
-        ps.p = 0;
-        ps.t = 0;
-        ps.m = log_n;
-        ps.rest = 0;
-        ps.log_in = log_in;
-        ps.pre = pre;
-        ps.post = post;
-        return launch_pass<1, true>(ctx, in, out, tab, ps, pre_c, post_c);
-    }
-    size_t bytes = sizeof(Fr) << log_n;
-    B2_TRY(scratch_reserve(ctx, ctx->ntt_work, bytes));
-    Fr* W = (Fr*)ctx->ntt_work.p;
-    uint32_t t = 0;
-    for (uint32_t p = 0; p < ps.P; ++p) {
-        ps.p = p;
-        ps.t = t;
-        ps.m = ps.dig[p];
-        ps.rest = log_n - t - ps.m;
-        ps.log_in = (p == 0) ? log_in : log_n;
-        ps.pre = (p == 0) ? pre : 0;
-        ps.post = (p + 1 == ps.P) ? post : 0;
-        if (p + 1 < ps.P)
-            B2_TRY((launch_pass<8, false>(ctx, p == 0 ? in : W, W, tab, ps, pre_c, post_c)));
-        else
-            B2_TRY((launch_pass<8, true>(ctx, W, out, tab, ps, pre_c, post_c)));
-        t += ps.m;
-    }
-    return B200ZK_OK;
+Fr host_root_of_unity(uint32_t log_n) {  // halo2curves Fr::ROOT_OF_UNITY^(2^(28 - log_n)): EvaluationDomain's omega of a 2^log_n domain
+    Fr w;
+    const uint32_t v[8] = {0xb639feb8u, 0x9632c7c5u, 0x0d0ff299u, 0x985ce340u, 0x01b0ecd8u, 0xb2dd8800u, 0x6d98ce29u, 0x1d69070du};
+    for (int i = 0; i < 8; ++i) w.l.v[i] = v[i];
+    for (uint32_t i = log_n; i < 28; ++i) w = w.sqr();
+    return w;
+}
+
+// Part `part` of the extended coset zeta * <w_ext> (2^ext_k points), i.e. the n = 2^k points g * w^i, g = zeta * w_ext^part:
+//   forward (coeff_to_extended_part):  out[i] = sum_m in[m] g^m w^(im)           (pre-scale by zeta^(m mod 3) w_ext^(part*m))
+//   inverse (the first half of extended_parts_to_coeff):  out[m] = scale * g^-m * n^-1 * sum_i in[i] w^(-im)
+// Both are one n-point transform with the twist fused into its first load / last store.  in == out is allowed.
+int32_t ntt_part_run(b200zk_ctx* ctx, const Fr* in, Fr* out, uint32_t k, uint32_t ext_k, uint32_t part, bool inverse,
+                     const Fr& scale) {
+    Fr u = host_root_of_unity(ext_k);
+    if (inverse) u = u.inv();
+    const Fr* tab = nullptr;
+    B2_TRY(ntt_get_table(ctx, u, ext_k, &tab));
+    PartTwist tw;
+    tw.wtab = tab + (1ull << (ext_k - 1));
+    tw.mask = (1ull << ext_k) - 1;
+    tw.part = part;
+    tw.pre = !inverse;
+    tw.post = inverse;
+    Fr zeta = host_zeta(), zeta2 = zeta.sqr();
+    Fr3 pre_c, post_c;
+    pre_c.c[0] = Fr::one();
+    pre_c.c[1] = zeta;
+    pre_c.c[2] = zeta2;
+    Fr s = scale;
+    if (inverse)
+        for (uint32_t i = 0; i < k; ++i) s = host_halve(s);
+    post_c.c[0] = s;
+    post_c.c[1] = s * zeta2;
+    post_c.c[2] = s * zeta;
+    return ntt_passes(ctx, in, k, out, k, tab, inverse ? 0 : 1, inverse ? 1 : 0, pre_c, post_c, tw);
 }
 
 }  // namespace b200zk

@@ -409,6 +409,76 @@ int32_t lincomb_run(b200zk_ctx* ctx, const void* const* polys, const Fr* scalars
     return B200ZK_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ quotient from coset parts
+// e_r[m] (r < J parts of n coefficients, part-major) -> h_j[m] = zeta^(-n j) J^-1 sum_r w_J^(-r j) e_r[m], j < n_pieces:
+// a J-point inverse DFT per coefficient index, held in registers (radix-2 DIT, bit-reversed loads).  HBM-bound:
+// (J + n_pieces) * 32 B per index.  out may equal parts (every index is read in full before its pieces are written).
+struct PartsDft {
+    Fr tw[8];   // w_J^-k, k < J/2
+    Fr sc[16];  // zeta^(-n j) / J
+};
+
+template <int J>
+__global__ void __launch_bounds__(128) parts_recombine_kernel(const Fr* parts, uint64_t n, uint32_t n_pieces, PartsDft D, Fr* out) {
+    constexpr int LOGJ = J == 1 ? 0 : J == 2 ? 1 : J == 4 ? 2 : J == 8 ? 3 : 4;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t m = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; m < n; m += stride) {
+        Fr a[J];
+#pragma unroll
+        for (int r = 0; r < J; ++r) {
+            int br = 0;
+#pragma unroll
+            for (int b = 0; b < LOGJ; ++b) br |= ((r >> b) & 1) << (LOGJ - 1 - b);
+            a[br] = q_ld(parts + (uint64_t)r * n + m);
+        }
+#pragma unroll
+        for (int len = 2; len <= J; len <<= 1) {
+#pragma unroll
+            for (int s0 = 0; s0 < J; s0 += len) {
+#pragma unroll
+                for (int q = 0; q < len / 2; ++q) {
+                    Fr u = a[s0 + q], v = a[s0 + q + len / 2];
+                    if (q) v = v * D.tw[q * (J / len)];
+                    a[s0 + q] = u + v;
+                    a[s0 + q + len / 2] = u - v;
+                }
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < J; ++j)
+            if ((uint32_t)j < n_pieces) q_st(out + (uint64_t)j * n + m, a[j] * D.sc[j]);
+    }
+}
+
+int32_t parts_recombine_run(b200zk_ctx* ctx, const Fr* parts, uint32_t k, uint32_t log_j, uint32_t n_pieces, const Fr& zeta_n_inv,
+                            const Fr& w_j_inv, const Fr& j_inv, Fr* out) {
+    const uint64_t n = 1ull << k;
+    const uint32_t J = 1u << log_j;
+    PartsDft D;
+    Fr w = Fr::one();
+    for (uint32_t i = 0; i < 8; ++i) {
+        D.tw[i] = w;
+        w = w * w_j_inv;
+    }
+    Fr sc = j_inv;
+    for (uint32_t j = 0; j < 16; ++j) {
+        D.sc[j] = sc;
+        sc = sc * zeta_n_inv;
+    }
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>((n + 127) / 128, (uint64_t)ctx->sm_count * 16);
+    ProfScope ps_(ctx, PROF_POLY);
+    switch (J) {
+        case 1: parts_recombine_kernel<1><<<blocks, 128, 0, ctx->stream>>>(parts, n, n_pieces, D, out); break;
+        case 2: parts_recombine_kernel<2><<<blocks, 128, 0, ctx->stream>>>(parts, n, n_pieces, D, out); break;
+        case 4: parts_recombine_kernel<4><<<blocks, 128, 0, ctx->stream>>>(parts, n, n_pieces, D, out); break;
+        case 8: parts_recombine_kernel<8><<<blocks, 128, 0, ctx->stream>>>(parts, n, n_pieces, D, out); break;
+        case 16: parts_recombine_kernel<16><<<blocks, 128, 0, ctx->stream>>>(parts, n, n_pieces, D, out); break;
+        default: return fail(ctx, B200ZK_E_UNSUPPORTED, "extended_parts_to_coeff: J = %u is not supported", J);
+    }
+    B2_LAUNCH_CHECK(ctx);
+    return B200ZK_OK;
+}
+
 }  // namespace b200zk
 
 using namespace b200zk;
@@ -595,12 +665,14 @@ int32_t b200zk_graph_evaluate(b200zk_ctx* ctx, const b200zk_graph* graph, const 
                                       log_size <= 30 ? (1ull << log_size) : 0);
 }
 
-int32_t b200zk_graph_evaluate_rows(b200zk_ctx* ctx, const b200zk_graph* graph, const void* const* fixed_dev, uint32_t n_fixed,
+}  // extern "C"
+
+// rows [row_first, +row_count) of a domain of 2^log_size points x_zeta * w^row (w read from x_omega32 when the program uses x)
+static int32_t graph_evaluate_impl(b200zk_ctx* ctx, const b200zk_graph* graph, const void* const* fixed_dev, uint32_t n_fixed,
                                    const void* const* advice_dev, uint32_t n_advice, const void* const* instance_dev, uint32_t n_instance,
                                    const void* challenges32, uint32_t n_challenges, const void* beta32, const void* gamma32,
-                                   const void* theta32, const void* y32, const void* extended_omega32, void* values_dev, uint32_t log_size,
-                                   int32_t rot_scale, uint64_t row_first, uint64_t row_count) {
-    CHECK_CTX(ctx);
+                                   const void* theta32, const void* y32, const void* x_omega32, void* values_dev, uint32_t log_size,
+                                   int32_t rot_scale, uint64_t row_first, uint64_t row_count, const Fr& x_zeta) {
     if (!graph) return fail(ctx, B200ZK_E_INVALID, "graph_evaluate: null graph");
     if (log_size > 30) return fail(ctx, B200ZK_E_INVALID, "graph_evaluate: log_size = %u > 30", log_size);
     if (row_first > (1ull << log_size) || row_count > (1ull << log_size) - row_first)
@@ -649,12 +721,12 @@ int32_t b200zk_graph_evaluate_rows(b200zk_ctx* ctx, const b200zk_graph* graph, c
     L.uses_x = P.uses_x;
     L.uses_prev = P.uses_prev;
     L.xtab = nullptr;
-    L.zeta = host_zeta();
+    L.zeta = x_zeta;
     L.row_first = row_first;
     L.row_count = row_count;
     if (P.uses_x && log_size) {
         Fr w;
-        B2_TRY(read_fr(ctx, extended_omega32, &w));
+        B2_TRY(read_fr(ctx, x_omega32, &w));
         const Fr* tab = nullptr;
         B2_TRY(ntt_get_table(ctx, w, log_size, &tab));
         L.xtab = tab + (size >> 1);
@@ -665,6 +737,35 @@ int32_t b200zk_graph_evaluate_rows(b200zk_ctx* ctx, const b200zk_graph* graph, c
     if (P.n_rotations) B2_CUDA(ctx, cudaMemcpyAsync(graph->dev_rot, rot_off.data(), sizeof(uint32_t) * P.n_rotations, cudaMemcpyHostToDevice, ctx->stream));
     if (graph->cols_cap) B2_CUDA(ctx, cudaMemcpyAsync(graph->dev_cols, cols.data(), sizeof(void*) * graph->cols_cap, cudaMemcpyHostToDevice, ctx->stream));
     return graph_evaluate_run(ctx, graph, L);
+}
+
+extern "C" {
+
+int32_t b200zk_graph_evaluate_rows(b200zk_ctx* ctx, const b200zk_graph* graph, const void* const* fixed_dev, uint32_t n_fixed,
+                                   const void* const* advice_dev, uint32_t n_advice, const void* const* instance_dev, uint32_t n_instance,
+                                   const void* challenges32, uint32_t n_challenges, const void* beta32, const void* gamma32,
+                                   const void* theta32, const void* y32, const void* extended_omega32, void* values_dev, uint32_t log_size,
+                                   int32_t rot_scale, uint64_t row_first, uint64_t row_count) {
+    CHECK_CTX(ctx);
+    return graph_evaluate_impl(ctx, graph, fixed_dev, n_fixed, advice_dev, n_advice, instance_dev, n_instance, challenges32, n_challenges,
+                               beta32, gamma32, theta32, y32, extended_omega32, values_dev, log_size, rot_scale, row_first, row_count,
+                               host_zeta());
+}
+
+int32_t b200zk_graph_evaluate_part(b200zk_ctx* ctx, const b200zk_graph* graph, const void* const* fixed_dev, uint32_t n_fixed,
+                                   const void* const* advice_dev, uint32_t n_advice, const void* const* instance_dev, uint32_t n_instance,
+                                   const void* challenges32, uint32_t n_challenges, const void* beta32, const void* gamma32,
+                                   const void* theta32, const void* y32, uint32_t k, uint32_t extended_k, uint32_t part, void* values_dev) {
+    CHECK_CTX(ctx);
+    B2_TRY(check_part_args(ctx, "graph_evaluate_part", k, extended_k, part));
+    // part r is the coset g_r * <w> of the n-th roots, g_r = zeta * w_ext^r: rotations move within the part (rot_scale 1)
+    Guard g(ctx);
+    const Fr w = host_root_of_unity(k);
+    Fr g_r = host_zeta(), w_ext = host_root_of_unity(extended_k);
+    for (uint32_t b = part; b; b >>= 1, w_ext = w_ext.sqr())
+        if (b & 1) g_r = g_r * w_ext;
+    return graph_evaluate_impl(ctx, graph, fixed_dev, n_fixed, advice_dev, n_advice, instance_dev, n_instance, challenges32, n_challenges,
+                               beta32, gamma32, theta32, y32, &w, values_dev, k, 1, 0, 1ull << k, g_r);
 }
 
 }  // extern "C"

@@ -5,7 +5,8 @@
 // halo2_proofs 1.1.0 (scroll-tech/halo2 @ e5ddf67, pin /root/reference/Cargo.lock:1886-1888):
 //
 //   halo2_b200::arithmetic::best_multiexp / best_fft / eval_polynomial / kate_division   (src/arithmetic.rs)
-//   halo2_b200::EvaluationDomain::{new_, lagrange_to_coeff, coeff_to_extended, extended_to_coeff}  (src/poly/domain.rs)
+//   halo2_b200::EvaluationDomain::{new_, lagrange_to_coeff, coeff_to_extended, extended_to_coeff}  (src/poly/domain.rs),
+//     plus coeff_to_extended_part / extended_parts_to_coeff: the extended coset as J parts of n points
 //   halo2_b200::ParamsKZG::{setup, read_custom, write_custom, commit, commit_lagrange, downsize-less accessors}
 //                                                                                    (src/poly/kzg/commitment.rs)
 // A Rust panic (assert_eq!, unwrap) is mirrored by throwing halo2_b200::Panic.  Types are layout-identical to
@@ -184,6 +185,37 @@ class EvaluationDomain {
         b.check(b200zk_ntt_fr(b.ctx(), a.data(), extended_k, &extended_omega_inv, 1, B200ZK_COSET_POST), "extended_to_coeff");
         a.resize((size_t)(n * quotient_poly_degree));  // truncate to the quotient degree
         return a;
+    }
+    // The extended coset as J = 2^(extended_k - k) parts of n points, part r = zeta * extended_omega^r * <omega>:
+    // coeff_to_extended(a)[part + J*i] for i < n
+    std::vector<Fr> coeff_to_extended_part(const std::vector<Fr>& a, uint32_t part) const {
+        if (a.size() != n) throw Panic("assertion failed: a.values.len() == 1 << self.k");
+        std::vector<Fr> out(n);
+        auto& b = Backend::get();
+        void* dev = nullptr;
+        b.check(b200zk_buf_alloc(b.ctx(), 32 * n, &dev), "coeff_to_extended_part");
+        const void* in = a.data();
+        int32_t rc = b200zk_coeff_to_extended_parts(b.ctx(), &in, 1, k, extended_k, part, &dev);
+        if (rc == B200ZK_OK) rc = b200zk_buf_download(b.ctx(), out.data(), dev, 32 * n);
+        b200zk_buf_free(b.ctx(), dev);
+        b.check(rc, "coeff_to_extended_part");
+        return out;
+    }
+    // extended_to_coeff (after divide_by_vanishing_poly when asked) of the extended coset given part-major: parts[r * n + i] is
+    // row r + J*i.  Returns the n * quotient_poly_degree coefficients, as extended_to_coeff does.
+    std::vector<Fr> extended_parts_to_coeff(const std::vector<Fr>& parts, bool divide_by_vanishing) const {
+        if (parts.size() != (size_t(1) << extended_k)) throw Panic("assertion failed: a.values.len() == self.extended_len()");
+        std::vector<Fr> out((size_t)(n * quotient_poly_degree));
+        auto& b = Backend::get();
+        void* dev = nullptr;
+        b.check(b200zk_buf_alloc(b.ctx(), 32 * parts.size(), &dev), "extended_parts_to_coeff");
+        int32_t rc = b200zk_buf_upload(b.ctx(), dev, parts.data(), 32 * parts.size());
+        if (rc == B200ZK_OK)
+            rc = b200zk_extended_parts_to_coeff(b.ctx(), dev, k, extended_k, (uint32_t)quotient_poly_degree, divide_by_vanishing ? 1 : 0, dev);
+        if (rc == B200ZK_OK) rc = b200zk_buf_download(b.ctx(), out.data(), dev, 32 * out.size());
+        b200zk_buf_free(b.ctx(), dev);
+        b.check(rc, "extended_parts_to_coeff");
+        return out;
     }
 };
 
@@ -446,6 +478,28 @@ class GraphEvaluator {
                                       (uint32_t)ti.size(), challenges.data(), (uint32_t)challenges.size(), &beta, &gamma, &theta, &y,
                                       &dom.extended_omega, values.ptr(), dom.extended_k, rot_scale),
                 "GraphEvaluator::evaluate");
+    }
+    // the same on the n rows of one part of the extended coset (columns hold that part's values, rotations wrap within it)
+    void evaluate_part(DeviceColumn& values, const EvaluationDomain& dom, uint32_t part, const std::vector<const DeviceColumn*>& fixed,
+                       const std::vector<const DeviceColumn*>& advice, const std::vector<const DeviceColumn*>& instance,
+                       const std::vector<Fr>& challenges, const Fr& beta, const Fr& gamma, const Fr& theta, const Fr& y) {
+        auto& b = Backend::get();
+        if (values.len() != dom.n) throw Panic("GraphEvaluator::evaluate_part: values must cover one part (n rows)");
+        if (!graph_)
+            b.check(b200zk_graph_create(b.ctx(), calcs_.data(), (uint32_t)calcs_.size(), parts_.data(), (uint32_t)parts_.size(),
+                                        constants_.data(), (uint32_t)constants_.size(), rotations_.data(), (uint32_t)rotations_.size(),
+                                        &graph_),
+                    "GraphEvaluator::compile");
+        auto table = [](const std::vector<const DeviceColumn*>& v) {
+            std::vector<const void*> t;
+            for (auto* c : v) t.push_back(c->ptr());
+            return t;
+        };
+        auto tf = table(fixed), ta = table(advice), ti = table(instance);
+        b.check(b200zk_graph_evaluate_part(b.ctx(), graph_, tf.data(), (uint32_t)tf.size(), ta.data(), (uint32_t)ta.size(), ti.data(),
+                                           (uint32_t)ti.size(), challenges.data(), (uint32_t)challenges.size(), &beta, &gamma, &theta, &y,
+                                           dom.k, dom.extended_k, part, values.ptr()),
+                "GraphEvaluator::evaluate_part");
     }
     void release() {
         if (graph_) b200zk_graph_destroy(Backend::get().ctx(), graph_);

@@ -529,6 +529,7 @@ struct Program {  // a GraphEvaluator program in the ABI's (= upstream's) form
     std::vector<int32_t> rotations;
 };
 using Poly = std::vector<Fr>;
+struct ProvingKey;
 
 struct Ops {
     virtual ~Ops() = default;
@@ -551,6 +552,12 @@ struct Ops {
     // mv_lookup phi(X) running sum
     virtual Poly logup_running_sum(const std::vector<const Poly*>& inputs, const Poly& table, const Poly& m, const Fr& beta,
                                    const Fr& phi_init) = 0;
+    // evaluate_h (gates, permutation, lookups folded with y) + divide_by_vanishing_poly + extended_to_coeff: the
+    // n * quotient_poly_degree coefficients of h.  Columns in coefficient form, in the programs' table order:
+    // advice = [cs advice..., z sets..., (m, phi) per lookup].  The default works on full extended cosets (defined below).
+    virtual Poly quotient(const ProvingKey& pk, const EvaluationDomain& dom, const std::vector<const Poly*>& advice,
+                          const std::vector<const Poly*>& instance, const std::vector<Fr>& challenges, const Fr& beta, const Fr& gamma,
+                          const Fr& theta, const Fr& y);
 };
 
 // The product: every operation through the C ABI.  Host vectors in and out (the ABI stages them); the quotient-construction
@@ -636,9 +643,20 @@ class DeviceOps : public Ops {
         return phi.to_host();
     }
 
+    // Part by part (DESIGN.md "Quotient construction"): every coefficient-form column is uploaded once; for each of the J
+    // parts of the extended coset, all columns are transformed into one reused set of n-row scratch columns and the programs
+    // chain into slot r of one 2^extended_k buffer; one b200zk_extended_parts_to_coeff divides by X^n - 1 and recombines.
+    // No column is ever held at extended size.  Domains with more parts than the kernels support take the full-coset path.
+    Poly quotient(const ProvingKey& pk, const EvaluationDomain& dom, const std::vector<const Poly*>& advice,
+                  const std::vector<const Poly*>& instance, const std::vector<Fr>& challenges, const Fr& beta, const Fr& gamma,
+                  const Fr& theta, const Fr& y) override;
+    // device bytes the last quotient() held at its peak (columns, scratch and the part buffer)
+    size_t quotient_peak_bytes() const { return quotient_peak_; }
+
   private:
     ParamsKZG& params_;
     const EvaluationDomain& dom_;
+    size_t quotient_peak_ = 0;
 };
 
 // ------------------------------------------------------------------------------------------------ keys
@@ -670,6 +688,7 @@ struct VerifyingKey {
 struct ProvingKey {
     VerifyingKey vk;
     Poly l0, l_last, l_active_row;                       // extended cosets
+    Poly l0_poly, l_last_poly, l_active_row_poly;        // the same in coefficient form
     std::vector<Poly> fixed_values, fixed_polys, fixed_cosets;
     std::vector<Poly> sigma_values, sigma_polys, sigma_cosets;
     Program gates;                                        // custom gates folded with y
@@ -716,6 +735,112 @@ inline AuxLayout aux_layout(const ConstraintSystem& cs) {
     uint32_t chunk = cs.permutation_chunk_len();
     a.n_sets = cs.permutation.empty() ? 0 : (uint32_t)((cs.permutation.size() + chunk - 1) / chunk);
     return a;
+}
+
+// evaluate_h on full extended cosets: every column's coset, the programs over the whole extended domain, the 1/(X^n - 1) column
+inline Poly Ops::quotient(const ProvingKey& pk, const EvaluationDomain& dom, const std::vector<const Poly*>& advice,
+                          const std::vector<const Poly*>& instance, const std::vector<Fr>& challenges, const Fr& beta, const Fr& gamma,
+                          const Fr& theta, const Fr& y) {
+    const ConstraintSystem& cs = pk.vk.cs;
+    const uint64_t n = dom.n;
+    std::vector<Poly> advice_cosets, instance_cosets;
+    for (auto* c : advice) advice_cosets.push_back(coeff_to_extended(*c));
+    for (auto* c : instance) instance_cosets.push_back(coeff_to_extended(*c));
+    const size_t ext_n = (size_t)1 << dom.extended_k;
+    Poly h_ext(ext_n, f_zero());
+    std::vector<const Poly*> fixed_tab, advice_tab, instance_tab;
+    for (auto& c : pk.fixed_cosets) fixed_tab.push_back(&c);
+    fixed_tab.push_back(&pk.l0);
+    fixed_tab.push_back(&pk.l_last);
+    fixed_tab.push_back(&pk.l_active_row);
+    for (auto& c : pk.sigma_cosets) fixed_tab.push_back(&c);
+    for (auto& c : advice_cosets) advice_tab.push_back(&c);
+    for (auto& c : instance_cosets) instance_tab.push_back(&c);
+    if (!pk.gates.calcs.empty()) graph_evaluate(pk.gates, fixed_tab, advice_tab, instance_tab, challenges, beta, gamma, theta, y, h_ext);
+    if (!cs.permutation.empty()) graph_evaluate(pk.permutation, fixed_tab, advice_tab, instance_tab, challenges, beta, gamma, theta, y, h_ext);
+    for (auto& prog : pk.lookups) graph_evaluate(prog, fixed_tab, advice_tab, instance_tab, challenges, beta, gamma, theta, y, h_ext);
+    {   // EvaluationDomain::divide_by_vanishing_poly: (zeta * w_ext^i)^n - 1 takes 2^(extended_k - k) distinct values
+        const size_t period = (size_t)1 << (dom.extended_k - dom.k);
+        std::vector<Fr> t_inv(period);
+        Fr zn = f_pow(dom.g_coset, n), wn = f_pow(dom.extended_omega, n), cur = zn;
+        for (size_t i = 0; i < period; ++i) { t_inv[i] = f_inv(f_sub(cur, f_one())); cur = f_mul(cur, wn); }
+        Poly t_col(ext_n);
+        for (size_t i = 0; i < ext_n; ++i) t_col[i] = t_inv[i % period];
+        h_ext = poly_mul(h_ext, t_col);
+    }
+    return extended_to_coeff(std::move(h_ext));  // n * quotient_poly_degree coefficients
+}
+
+inline Poly DeviceOps::quotient(const ProvingKey& pk, const EvaluationDomain& dom, const std::vector<const Poly*>& advice,
+                                const std::vector<const Poly*>& instance, const std::vector<Fr>& challenges, const Fr& beta,
+                                const Fr& gamma, const Fr& theta, const Fr& y) {
+    const uint32_t k = dom.k, ek = dom.extended_k;
+    if (ek - k > 4) return Ops::quotient(pk, dom, advice, instance, challenges, beta, gamma, theta, y);  // J > 16 parts
+    const uint32_t J = 1u << (ek - k);
+    const uint64_t n = dom.n;
+    auto& be = Backend::get();
+    size_t held = 0;
+    quotient_peak_ = 0;
+    auto hold = [&](uint64_t elems) { held += 32 * (size_t)elems; quotient_peak_ = std::max(quotient_peak_, held); };
+    // the columns in the programs' table order (fixed | advice | instance), coefficient form, each uploaded once
+    std::vector<const Poly*> cols;
+    for (auto& c : pk.fixed_polys) cols.push_back(&c);
+    cols.push_back(&pk.l0_poly);
+    cols.push_back(&pk.l_last_poly);
+    cols.push_back(&pk.l_active_row_poly);
+    for (auto& c : pk.sigma_polys) cols.push_back(&c);
+    const uint32_t n_fixed = (uint32_t)cols.size();
+    cols.insert(cols.end(), advice.begin(), advice.end());
+    cols.insert(cols.end(), instance.begin(), instance.end());
+    const uint32_t n_advice = (uint32_t)advice.size(), n_instance = (uint32_t)instance.size();
+    std::vector<DeviceColumn> coeff, part_cols;
+    coeff.reserve(cols.size());
+    part_cols.reserve(cols.size());
+    std::vector<const void*> coeff_ptrs;
+    std::vector<void*> part_ptrs;
+    for (auto* c : cols) {
+        coeff.emplace_back(*c);
+        hold(n);
+        coeff_ptrs.push_back(coeff.back().ptr());
+    }
+    for (size_t i = 0; i < cols.size(); ++i) {
+        part_cols.emplace_back((size_t)n);
+        hold(n);
+        part_ptrs.push_back(part_cols.back().ptr());
+    }
+    DeviceColumn parts((size_t)J * n);
+    hold((uint64_t)J * n);
+    struct Graphs {  // the evaluate_h programs, released on every exit
+        std::vector<b200zk_graph*> g;
+        ~Graphs() { for (auto* h : g) b200zk_graph_destroy(Backend::get().ctx(), h); }
+    } graphs;
+    auto compile = [&](const Program& p) {
+        b200zk_graph* g = nullptr;
+        be.check(b200zk_graph_create(be.ctx(), p.calcs.data(), (uint32_t)p.calcs.size(), p.parts.data(), (uint32_t)p.parts.size(),
+                                     p.constants.data(), (uint32_t)p.constants.size(), p.rotations.data(), (uint32_t)p.rotations.size(), &g),
+                 "graph_create");
+        graphs.g.push_back(g);
+    };
+    if (!pk.gates.calcs.empty()) compile(pk.gates);
+    if (!pk.vk.cs.permutation.empty()) compile(pk.permutation);
+    for (auto& prog : pk.lookups) compile(prog);
+    const Poly zeros(n, f_zero());
+    const void* const* tf = (const void* const*)part_ptrs.data();
+    for (uint32_t r = 0; r < J; ++r) {
+        be.check(b200zk_coeff_to_extended_parts(be.ctx(), coeff_ptrs.data(), (uint32_t)cols.size(), k, ek, r, part_ptrs.data()),
+                 "coeff_to_extended_parts");
+        void* slot = (char*)parts.ptr() + 32 * (size_t)r * n;
+        be.check(b200zk_buf_upload(be.ctx(), slot, zeros.data(), 32 * n), "quotient: clear part");
+        for (auto* g : graphs.g)
+            be.check(b200zk_graph_evaluate_part(be.ctx(), g, tf, n_fixed, tf + n_fixed, n_advice, tf + n_fixed + n_advice, n_instance,
+                                                challenges.data(), (uint32_t)challenges.size(), &beta, &gamma, &theta, &y, k, ek, r, slot),
+                     "graph_evaluate_part");
+    }
+    const uint64_t pieces = dom.quotient_poly_degree;
+    be.check(b200zk_extended_parts_to_coeff(be.ctx(), parts.ptr(), k, ek, (uint32_t)pieces, 1, parts.ptr()), "extended_parts_to_coeff");
+    Poly h(pieces * n);
+    be.check(b200zk_buf_download(be.ctx(), h.data(), parts.ptr(), 32 * pieces * n), "quotient: download");
+    return h;
 }
 
 // keygen_vk + keygen_pk: fixed columns (Lagrange values), the permutation assembly; polynomials and cosets through `ops`
@@ -772,11 +897,17 @@ inline ProvingKey keygen(Ops& ops, const EvaluationDomain& dom, ConstraintSystem
     l0[0] = f_one();
     for (uint64_t r = n - bf; r < n; ++r) l_blind[r] = f_one();
     l_last[n - bf - 1] = f_one();
-    pk.l0 = ops.coeff_to_extended(ops.lagrange_to_coeff(l0));
-    Poly lb = ops.coeff_to_extended(ops.lagrange_to_coeff(l_blind));
-    pk.l_last = ops.coeff_to_extended(ops.lagrange_to_coeff(l_last));
+    pk.l0_poly = ops.lagrange_to_coeff(l0);
+    pk.l0 = ops.coeff_to_extended(pk.l0_poly);
+    Poly lb_poly = ops.lagrange_to_coeff(l_blind);
+    Poly lb = ops.coeff_to_extended(lb_poly);
+    pk.l_last_poly = ops.lagrange_to_coeff(l_last);
+    pk.l_last = ops.coeff_to_extended(pk.l_last_poly);
     pk.l_active_row.resize(pk.l0.size());
     for (size_t i = 0; i < pk.l0.size(); ++i) pk.l_active_row[i] = f_sub(f_sub(f_one(), pk.l_last[i]), lb[i]);
+    // 1 - l_last - l_blind in coefficient form (the constant 1 is coefficient 0): its coset is l_active_row exactly
+    pk.l_active_row_poly.resize(n);
+    for (uint64_t i = 0; i < n; ++i) pk.l_active_row_poly[i] = f_sub(f_sub(i == 0 ? f_one() : f_zero(), pk.l_last_poly[i]), lb_poly[i]);
     pk.vk.transcript_repr = vk_transcript_repr(pk.vk);
 
     // ---- Evaluator::new: the programs of evaluate_h
@@ -960,20 +1091,19 @@ inline ProofArtifacts create_proof(Ops& ops, const EvaluationDomain& dom, const 
 
     // 0. vk and instances into the transcript (vk.hash_into; instance values as common scalars -- KZG: query_instance = false)
     tr.common_scalar(pk.vk.transcript_repr);
-    std::vector<Poly> instance_polys, instance_cosets;
+    std::vector<Poly> instance_polys;
     for (auto& inst : instances) {
         if (inst.size() != n) throw Panic("create_proof: instance column length");
         for (uint64_t r = u; r < n; ++r)
             if (!f_is_zero(inst[r])) throw Panic("create_proof: instance values beyond the usable rows");
         instance_polys.push_back(ops.lagrange_to_coeff(inst));
-        instance_cosets.push_back(ops.coeff_to_extended(instance_polys.back()));
     }
     for (auto& inst : instances)
         for (uint64_t r = 0; r < u; ++r) tr.common_scalar(inst[r]);
 
     // 1. advice, phase by phase: witness, blinding rows, commitments (commit_lagrange), the phase's challenges; then the
-    //    coefficient form and the extended cosets of every column
-    std::vector<Poly> advice(cs.num_advice, Poly(n, f_zero())), advice_polys, advice_cosets;
+    //    coefficient form of every column
+    std::vector<Poly> advice(cs.num_advice, Poly(n, f_zero())), advice_polys;
     std::vector<Fr> challenges(cs.challenge_phase.size(), f_zero());
     for (uint32_t phase = 0; phase < cs.num_phases(); ++phase) {
         std::vector<Poly> work = advice;
@@ -990,10 +1120,7 @@ inline ProofArtifacts create_proof(Ops& ops, const EvaluationDomain& dom, const 
         for (size_t i = 0; i < challenges.size(); ++i)
             if (cs.challenge_phase[i] == phase) challenges[i] = tr.squeeze_challenge();
     }
-    for (auto& col : advice) {
-        advice_polys.push_back(ops.lagrange_to_coeff(col));
-        advice_cosets.push_back(ops.coeff_to_extended(advice_polys.back()));
-    }
+    for (auto& col : advice) advice_polys.push_back(ops.lagrange_to_coeff(col));
     const Fr theta = tr.squeeze_challenge();
 
     // 2. lookups, first half (mv_lookup::Argument::prepare): compress with theta, count multiplicities, commit m
@@ -1042,7 +1169,7 @@ inline ProofArtifacts create_proof(Ops& ops, const EvaluationDomain& dom, const 
 
     // 3. permutation::Argument::commit: one grand product per column set, chained through z[u]
     const Fr delta = f_delta();
-    std::vector<Poly> z_values, z_polys, z_cosets;
+    std::vector<Poly> z_values, z_polys;
     if (!cs.permutation.empty()) {
         const uint32_t chunk = cs.permutation_chunk_len();
         Fr z_init = f_one(), delta_omega = f_one();
@@ -1061,10 +1188,7 @@ inline ProofArtifacts create_proof(Ops& ops, const EvaluationDomain& dom, const 
         }
         if (!(z_init == f_one())) throw Panic("permutation product does not close: the witness violates a copy constraint");
         for (auto& z : z_values) write_point(ops.commit_lagrange(z));
-        for (auto& z : z_values) {
-            z_polys.push_back(ops.lagrange_to_coeff(z));
-            z_cosets.push_back(ops.coeff_to_extended(z_polys.back()));
-        }
+        for (auto& z : z_values) z_polys.push_back(ops.lagrange_to_coeff(z));
     }
     // 4. lookups, second half (commit_grand_sum): phi running sum, blinded, committed
     for (auto& l : lk) {
@@ -1079,40 +1203,18 @@ inline ProofArtifacts create_proof(Ops& ops, const EvaluationDomain& dom, const 
     write_point(ops.commit(random_poly));
     const Fr y = tr.squeeze_challenge();
 
-    // 6. evaluate_h on the extended coset: gates, permutation, lookups folded with y; divide by X^n - 1
-    const size_t ext_n = (size_t)1 << dom.extended_k;
-    Poly h_ext(ext_n, f_zero());
-    std::vector<const Poly*> fixed_tab, advice_tab, instance_tab;
-    for (auto& c : pk.fixed_cosets) fixed_tab.push_back(&c);
-    fixed_tab.push_back(&pk.l0);
-    fixed_tab.push_back(&pk.l_last);
-    fixed_tab.push_back(&pk.l_active_row);
-    for (auto& c : pk.sigma_cosets) fixed_tab.push_back(&c);
-    for (auto& c : advice_cosets) advice_tab.push_back(&c);
-    for (auto& c : z_cosets) advice_tab.push_back(&c);
-    std::vector<Poly> lk_cosets;  // m, phi cosets per lookup
-    lk_cosets.reserve(2 * lk.size());
+    // 6. evaluate_h: gates, permutation, lookups folded with y; divided by X^n - 1; back to coefficients
+    std::vector<const Poly*> advice_tab, instance_tab;
+    for (auto& c : advice_polys) advice_tab.push_back(&c);
+    for (auto& c : z_polys) advice_tab.push_back(&c);
     for (auto& l : lk) {
         l.m_poly = ops.lagrange_to_coeff(l.m);
         l.phi_poly = ops.lagrange_to_coeff(l.phi);
-        lk_cosets.push_back(ops.coeff_to_extended(l.m_poly));
-        lk_cosets.push_back(ops.coeff_to_extended(l.phi_poly));
+        advice_tab.push_back(&l.m_poly);
+        advice_tab.push_back(&l.phi_poly);
     }
-    for (auto& c : lk_cosets) advice_tab.push_back(&c);
-    for (auto& c : instance_cosets) instance_tab.push_back(&c);
-    if (!pk.gates.calcs.empty()) ops.graph_evaluate(pk.gates, fixed_tab, advice_tab, instance_tab, challenges, beta, gamma, theta, y, h_ext);
-    if (!cs.permutation.empty()) ops.graph_evaluate(pk.permutation, fixed_tab, advice_tab, instance_tab, challenges, beta, gamma, theta, y, h_ext);
-    for (auto& prog : pk.lookups) ops.graph_evaluate(prog, fixed_tab, advice_tab, instance_tab, challenges, beta, gamma, theta, y, h_ext);
-    {   // EvaluationDomain::divide_by_vanishing_poly: (zeta * w_ext^i)^n - 1 takes 2^(extended_k - k) distinct values
-        const size_t period = (size_t)1 << (dom.extended_k - dom.k);
-        std::vector<Fr> t_inv(period);
-        Fr zn = f_pow(dom.g_coset, n), wn = f_pow(dom.extended_omega, n), cur = zn;
-        for (size_t i = 0; i < period; ++i) { t_inv[i] = f_inv(f_sub(cur, f_one())); cur = f_mul(cur, wn); }
-        Poly t_col(ext_n);
-        for (size_t i = 0; i < ext_n; ++i) t_col[i] = t_inv[i % period];
-        h_ext = ops.poly_mul(h_ext, t_col);
-    }
-    Poly h_coeffs = ops.extended_to_coeff(std::move(h_ext));  // n * quotient_poly_degree coefficients
+    for (auto& c : instance_polys) instance_tab.push_back(&c);
+    Poly h_coeffs = ops.quotient(pk, dom, advice_tab, instance_tab, challenges, beta, gamma, theta, y);  // n * quotient_poly_degree
     // vanishing::Committed::construct: pieces of n coefficients, each committed
     std::vector<Poly> h_pieces;
     for (size_t i = 0; i < dom.quotient_poly_degree; ++i) h_pieces.emplace_back(h_coeffs.begin() + i * n, h_coeffs.begin() + (i + 1) * n);
